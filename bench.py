@@ -3,7 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                   [--precision exact_tc|fast|exact] [--modality RGB|Flow] [--classes K] [--videos-per-gpu V]
-                  [--mode train|infer]
+                  [--mode train|infer] [--dump-outputs DIR]
   N>1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Default workload = BASELINE.json configs[1]: THUMOS14-shape synthetic, per GPU 4 videos x 8 proposals x 9 segments RGB
@@ -158,9 +158,9 @@ def metric_name(args):
 
 # ---- reference arm: the UNMODIFIED reference on the host CPU cores ------------------------------------------
 def run_reference(args):
-    """`--impl reference`: the reference's own CPU PyTorch implementation of the same step (baseline/_ref = a copy of the
-    reference's files made by __graft_entry__.build(); the oracle port only if that copy is missing), all host threads,
-    same configuration as our arm.  Rank 0 alone works."""
+    """`--impl reference`: the reference's own CPU PyTorch implementation of the same step (the checkout named by
+    SSNB_REFERENCE_DIR, baseline/ref_harness.py; the oracle port without it), all host threads, same configuration as our
+    arm.  Rank 0 alone works."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -246,7 +246,7 @@ def run_reference(args):
     value = units / mean
     cfg = config_dict(args, world=args.gpus)
     cfg.update({"precision": "f32 CPU", "note": "reference CPU PyTorch path (%s), rank 0 only, %d host threads" % (
-        "unmodified reference files from baseline/_ref" if kind == "reference" else "oracle restatement", cores)})
+        "unmodified reference checkout" if kind == "reference" else "oracle restatement", cores)})
     line = {"impl": "reference", "metric": metric_name(args), "value": value, "unit": "proposals/s", "n_gpus": args.gpus,
             "steps": len(times), "warmup": done_w, "steps_requested": args.steps, "ms_per_step": mean * 1e3,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -267,6 +267,25 @@ def config_dict(args, world):
 
 
 # ---- our arm ---------------------------------------------------------------------------------------------------
+DUMP_MAX_ELEMS = 1 << 20        # 4 MiB of float32 per array: a dump of at most nine arrays stays under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy (float64 stays float64, everything else float32), so that two builds
+    can be compared output for output.  An array of more than DUMP_MAX_ELEMS elements is replaced by a fixed sample of its
+    flattened elements (seeded: the same indices in every run)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
+
+
 def parse_timing(report):
     rows = []
     for ln in report.decode().splitlines():
@@ -295,8 +314,11 @@ def main():
     ap.add_argument("--no-second-mode", action="store_true", help="skip the side measurement of the other tensor-core mode")
     ap.add_argument("--grad-scale", type=float, default=4096.0)
     ap.add_argument("--no-graph", action="store_true", help="do not capture the training step in a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of --impl ours")
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
 
@@ -413,7 +435,7 @@ def main():
             return static_losses
         return graph_step
 
-    def measure_train(precision, steps, warmup, batches):
+    def measure_train(precision, steps, warmup, batches, dump_dir=None):
         model, flat_grad, opt, eager_step = build_train(precision)
         step, used_graph = eager_step, False
         if not args.no_graph:
@@ -425,6 +447,14 @@ def main():
                 torch.cuda.synchronize()
                 step, used_graph = eager_step, False
         ms_total, clocks, losses = timed_loop(step, batches, steps, warmup)
+        if dump_dir and rank == 0:
+            # the last timed step's results, before any later (eager) step overwrites them: the losses, the model outputs
+            # of fused_step (a replayed graph writes into the tensors captured in model.last_fused), the gradient and the
+            # parameters after the SGD update
+            lf = model.last_fused
+            dump_outputs(dump_dir, {"losses": losses, "act": lf["raw_act"], "comp": lf["raw_comp"], "reg": lf["raw_reg"],
+                                    "feat": lf["feat"], "course": lf["course"], "stpp": lf["stpp"], "grads": flat_grad,
+                                    "params": opt.flat_param})
         launches = count_launches(lambda: eager_step(batches[0])) * steps     # graph replays bypass the library's counter
         props_step = args.videos_per_gpu * PROPS * world
         res = {"value": props_step * steps / (ms_total / 1e3), "ms_per_step": ms_total / steps, "clocks": clocks,
@@ -435,7 +465,7 @@ def main():
         nb = 2   # distinct device-resident batches, alternated
         batches = [tuple(t.to(dev) for t in synth.synth_batch(args.videos_per_gpu, K, in_ch, seed=100 * rank + i)) for i in range(nb)]
         host_batches = [tuple(t.pin_memory() for t in synth.synth_batch(args.videos_per_gpu, K, in_ch, seed=100 * rank + i)) for i in range(nb)]
-        main, model, flat_grad, opt, eager_step = measure_train(args.precision, args.steps, args.warmup, batches)
+        main, model, flat_grad, opt, eager_step = measure_train(args.precision, args.steps, args.warmup, batches, args.dump_outputs)
         props_step = args.videos_per_gpu * PROPS * world
         frames_gpu = args.videos_per_gpu * PROPS * SEG
 
@@ -737,7 +767,9 @@ def run_infer(args, torch, dist, ssn_models, _lib, synth, dev, rank, world, loca
             return reorg.forward(out, ticks, scaling)
 
     model, reorg = build(args.precision)
-    ms_total, clocks, _ = timed_loop(lambda b: step_on(model, reorg, b), [video_dev], args.steps, args.warmup)
+    ms_total, clocks, scores = timed_loop(lambda b: step_on(model, reorg, b), [video_dev], args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("activity", "completeness", "regression"), scores)))
     launches = count_launches(lambda: step_on(model, reorg, video_dev)) * args.steps
     value = N * world * args.steps / (ms_total / 1e3)
     frames_s = T * crops * world * args.steps / (ms_total / 1e3)

@@ -66,11 +66,19 @@ def _worker(rank, world, port, out):
     dist.destroy_process_group()
 
 
+def free_port():
+    """a TCP port nothing on this host listens on (a fixed one can be taken by another job on a shared host)"""
+    import socket
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
+
 def test_dp_two_ranks_match_global_batch():
     world = 2
     mgr = mp.Manager()
     out = mgr.dict()
-    mp.spawn(_worker, args=(world, 29531, out), nprocs=world, join=True)
+    mp.spawn(_worker, args=(world, free_port(), out), nprocs=world, join=True)
     assert len(out) == world
     for r in range(world):
         assert out[r] < 1e-5, dict(out)

@@ -94,9 +94,10 @@ def test_bench_reference_arm_prints_contract_line():
     assert len(lines) == 1, lines
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["unit"] == "proposals/s" and d["higher_is_better"] is True and d["value"] > 0
-    # kind: the unmodified reference when build() vendored it into baseline/_ref, else the oracle port
-    vendored = os.path.exists(os.path.join(ROOT, "baseline", "_ref", "ssn_models.py"))
-    assert d["cpu_baseline"]["kind"] == ("reference" if vendored else "port")
+    # kind: the unmodified reference when SSNB_REFERENCE_DIR names a checkout of it, else the oracle port
+    ref = os.environ.get("SSNB_REFERENCE_DIR")
+    has_ref = bool(ref) and os.path.exists(os.path.join(ref, "ssn_models.py"))
+    assert d["cpu_baseline"]["kind"] == ("reference" if has_ref else "port")
     assert d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"] and d["steps"] == 1
     assert d["e2e"] == {"value": d["value"], "unit": "proposals/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "model" not in d["config"]
