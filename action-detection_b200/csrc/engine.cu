@@ -765,7 +765,6 @@ int ssnb_set_workspace(ssnb_handle h, void* dev_ptr, size_t bytes) {
         rc = umma_conv_bind_taps(h->umma_ctx, o.umma, xs, h->planes(o.out_val, false), h->F, Ck, c.cout, 4, dy, dx,
                                  (const __half*)(h->ws + h->s2d_w_off), (const float*)(h->ws + pk.bias), o.raw ? 0 : 1, &t);
         if (rc) return h->fail(rc, "tc conv1 bind: " + ssnb::thread_error());
-        if (!o.umma.p.v2) o.umma.enabled = false;
         if (use_wgrad_tc) {
           rc = umma_wgrad_bind_taps(h->umma_ctx, o.umma_wgrad, h->planes(o.out_val, true), xs, h->F, Ck, c.cout, 4, dy, dx,
                                     (float*)(h->ws + o.partial_off), 128);
@@ -787,7 +786,6 @@ int ssnb_set_workspace(ssnb_handle h, void* dev_ptr, size_t bytes) {
       rc = umma_conv_bind_dgrad(h->umma_ctx, o.umma_dgrad, dz, dxp, h->F, c.cin, c.cout, c.k, c.pad, (const __half*)(h->ws + pk.wf16),
                                 o.grad_accumulate, &tg);
       if (rc) return h->fail(rc, "tc bind_dgrad(" + c.id + "): " + ssnb::thread_error());
-      if (!o.umma_dgrad.p.v2) o.umma_dgrad.enabled = false;
       if (use_wgrad_tc) {
         rc = umma_wgrad_bind(h->umma_ctx, o.umma_wgrad, h->planes(o.out_val, true), h->planes(o.in_val, false), h->F, c.cin, c.cout, c.k, c.pad,
                              (float*)(h->ws + o.partial_off), o.tsplits, c.stride);
@@ -821,7 +819,6 @@ int ssnb_set_workspace(ssnb_handle h, void* dev_ptr, size_t bytes) {
                                   (const float*)(h->ws + fb.bias), &t);
         }
         if (rc) return h->fail(rc, "tc fused fwd bind(" + o3.id + "): " + ssnb::thread_error());
-        if (!fb.fwd.p.v2) continue;
         if (h->cfg.training) {
           View dredp = h->planes(o3.out_val, true); dredp.C = fb.c3r + fb.cdr;
           View d1p = fb.op1 >= 0 ? h->planes(h->ops[fb.op1].out_val, true) : dredp;
@@ -830,7 +827,6 @@ int ssnb_set_workspace(ssnb_handle h, void* dev_ptr, size_t bytes) {
           rc = umma_conv_bind_fused_dgrad(h->umma_ctx, fb.dgrad, d1p, dredp, dxp, h->F, fb.cx, fb.c1, fb.c3r + fb.cdr, (const __half*)(h->ws + fb.w_dg),
                                           od.grad_accumulate, &tg);
           if (rc) return h->fail(rc, "tc fused dgrad bind(" + o3.id + "): " + ssnb::thread_error());
-          if (!fb.dgrad.p.v2) continue;
           // zero the K padding of the concatenated data-gradient weights once (both planes); split_all_kernel never writes it
           if (cudaMemset(h->ws + fb.w_dg, 0, 2 * fb.w_dg_plane) != cudaSuccess) cudaGetLastError();
         }
@@ -972,8 +968,8 @@ int ssnb_set_workspace(ssnb_handle h, void* dev_ptr, size_t bytes) {
       if (c.kind == OP_GPOOL) c.dgrad_masks = true;
       else if (c.kind == OP_CONV && (c.fuse_role == 1 ? h->fused[c.fuse_block].enabled : (c.fuse_role == 0 && c.umma_dgrad.enabled))) {
         c.dgrad_masks = true;
-        const View yv = h->view((int)v, false);
-        if (c.fuse_role == 1) umma_conv_set_mask(h->umma_ctx, h->fused[c.fuse_block].dgrad, yv); else umma_conv_set_mask(h->umma_ctx, c.umma_dgrad, yv);
+        UmmaConvPlan& dg = c.fuse_role == 1 ? h->fused[c.fuse_block].dgrad : c.umma_dgrad;
+        if (int rc = umma_conv_set_mask(h->umma_ctx, dg, h->view((int)v, false))) return h->fail(rc, "mask fusion(" + c.id + "): " + ssnb::thread_error());
       }
     }
     for (Op& o : h->ops) {

@@ -1,14 +1,14 @@
 // tcgen05 implicit-GEMM convolution (sm_100a): host-side planning for both kernel generations, and the first-generation
-// kernel (per-tap A boxes), which still runs the four stride-2 forward layers (TMA element-stride boxes) and everything
-// under SSNB_V2=0.  All stride-1 layers run on umma_conv_v2.cu (halo boxes, CTA pairs, warp-uniform role loops).
+// kernel (per-tap A boxes), which runs the stride-2 forward layers.  Every stride-1 plan runs on umma_conv_v2.cu (halo
+// boxes, CTA pairs, warp-uniform role loops).
 //
-//   warp 0      : TMA producer   (A: 4-D activation box, B: 3-D weight box, SWIZZLE_128B)
+//   warp 0      : TMA producer   (A: 4-D activation box with TMA element stride 2, B: 3-D weight box, SWIZZLE_128B)
 //   warp 1      : TMEM allocator + MMA issuer (tcgen05.mma.cta_group::1.kind::f16, M=128, N=block_n)
-//   warps 2..9  : epilogue       (tcgen05.ld 32x32b -> bias/ReLU or accumulate/mask -> fp16 NHWC store); two warps per
-//                 TMEM lane quadrant take alternating 32-column groups (memory-level parallelism of the stores/loads)
+//   warps 2..9  : epilogue       (tcgen05.ld 32x32b -> bias/ReLU -> fp16 NHWC store, or the SSNB_EXACT_TC fp32 epilogue);
+//                 two warps per TMEM lane quadrant take alternating 32-column groups (memory-level parallelism of the stores)
 //
-// Rows of the M tile are the pixels of one TMA box (bw x bh x bf); taps shift the box origin and
-// rely on TMA's out-of-bounds zero fill for the convolution padding.
+// Rows of the M tile are the output pixels of one TMA box (bw x bh x bf); the box steps over the input with stride 2,
+// taps shift its origin and rely on TMA's out-of-bounds zero fill for the convolution padding.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -44,9 +44,8 @@ __device__ __forceinline__ TileCoord decode_tile(const UmmaConvParams& p, int ti
   return t;
 }
 
-// bias / accumulate / ReLU / ReLU-gradient mask on one 16-column chunk of an accumulator row, then fp16 store
-__device__ __forceinline__ void epilogue_chunk(const UmmaConvParams& p, const uint32_t* r, int col, uint4* dst, const uint4& o0,
-                                               const uint4& o1, const uint4& y0, const uint4& y1) {
+// bias / ReLU on one 16-column chunk of an accumulator row, then fp16 store
+__device__ __forceinline__ void epilogue_chunk(const UmmaConvParams& p, const uint32_t* r, int col, uint4* dst) {
   float v[16];
 #pragma unroll
   for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(r[j]);
@@ -54,30 +53,9 @@ __device__ __forceinline__ void epilogue_chunk(const UmmaConvParams& p, const ui
 #pragma unroll
     for (int j = 0; j < 16; ++j) v[j] += __ldg(p.bias + col + j);
   }
-  if (p.accumulate) {
-    const __half2* h0 = reinterpret_cast<const __half2*>(&o0);
-    const __half2* h1 = reinterpret_cast<const __half2*>(&o1);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      float2 a = __half22float2(h0[j]), b = __half22float2(h1[j]);
-      v[2 * j] += a.x; v[2 * j + 1] += a.y; v[8 + 2 * j] += b.x; v[8 + 2 * j + 1] += b.y;
-    }
-  }
   if (p.relu) {
 #pragma unroll
     for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j], 0.f);
-  }
-  if (p.mask_y) {
-    const __half2* a0 = reinterpret_cast<const __half2*>(&y0);
-    const __half2* a1 = reinterpret_cast<const __half2*>(&y1);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float2 ya = __half22float2(a0[j]), yb = __half22float2(a1[j]);
-      if (!(ya.x > 0.f)) v[2 * j] = 0.f;
-      if (!(ya.y > 0.f)) v[2 * j + 1] = 0.f;
-      if (!(yb.x > 0.f)) v[8 + 2 * j] = 0.f;
-      if (!(yb.y > 0.f)) v[8 + 2 * j + 1] = 0.f;
-    }
   }
   uint4 q0, q1;
   __half2* g0 = reinterpret_cast<__half2*>(&q0);
@@ -87,28 +65,22 @@ __device__ __forceinline__ void epilogue_chunk(const UmmaConvParams& p, const ui
   dst[0] = q0; dst[1] = q1;
 }
 
-// Direct variant of the epilogue (SSNB_EPI=0): every thread stores its own accumulator row, 32 bytes per 16 columns.
-// Epilogue role shared by the kernels: for every tile of this CTA wait for the accumulator, then TMEM -> registers ->
-// bias/ReLU (forward) or accumulate/mask (data gradient) -> fp16 NHWC stores.  Row r of the tile is pixel
-// (x, y, f) = (r % bw, (r / bw) % bh, r / (bw*bh)) in the classic layout and (r % bw, r / (bw*bf), (r / bw) % bf) in
-// the halo layout (rows ordered y-major, then frame, so that tap views have one uniform group stride).
-__device__ __forceinline__ void epilogue_loop_direct(const UmmaConvParams& p, uint32_t tmem_base, uint64_t* tfull_bar, uint64_t* tempty_bar,
+// Epilogue role: for every tile of this CTA wait for the accumulator, then TMEM -> registers -> bias/ReLU -> fp16 NHWC
+// stores (every thread stores its own accumulator row, 32 bytes per 16 columns).  Row r of the tile is output pixel
+// (x, y, f) = (r % bw, (r / bw) % bh, r / (bw*bh)).
+__device__ __forceinline__ void epilogue_loop(const UmmaConvParams& p, uint32_t tmem_base, uint64_t* tfull_bar, uint64_t* tempty_bar,
                                               int warp, int lane, int total_tiles, int tile0, int tstep) {
   const int quad = warp & 3;
   const int cpar = (warp - 2) >> 2;
   const int row = quad * 32 + lane;
-  int rw, rh, rf;
-  if (p.halo) { rw = row % p.bw; rf = (row / p.bw) % p.bf; rh = row / (p.bw * p.bf); }
-  else { rw = row % p.bw; rh = (row / p.bw) % p.bh; rf = row / (p.bw * p.bh); }
+  const int rw = row % p.bw, rh = (row / p.bw) % p.bh, rf = row / (p.bw * p.bh);
   uint32_t acc = 0, acc_phase = 0;
   for (int tile = tile0; tile < total_tiles; tile += tstep) {
     const TileCoord t = decode_tile(p, tile);
     const int w = t.w0 + rw, h = t.h0 + rh, f = t.f0 + rf;
-    const int os = p.out_stride;
-    const bool valid = (rf < p.bf) && (rh < p.bh) && (w < p.W) && (h < p.H) && (f < p.F) && (w % os == 0) && (h % os == 0);
-    const long long opix = (long long)(f * p.OH + h / os) * p.OW + w / os;
+    const bool valid = (rf < p.bf) && (w < p.W) && (h < p.H) && (f < p.F);
+    const long long opix = (long long)(f * p.H + h) * p.W + w;
     __half* orow = p.out + opix * p.out_pitch + p.out_coff;
-    __half* orow2 = p.out2 + opix * p.out2_pitch + p.out2_coff - p.n_split;
     mbar_wait(&tfull_bar[acc], acc_phase);
     tc_fence_after();
     const uint32_t taddr = tmem_base + acc * 256 + ((uint32_t)(quad * 32) << 16);
@@ -117,7 +89,6 @@ __device__ __forceinline__ void epilogue_loop_direct(const UmmaConvParams& p, ui
       float* orow32 = p.out32 + opix * p.out_pitch + p.out_coff;
       __half* hrow = p.out_hi ? p.out_hi + opix * p.out_pitch + p.out_coff : nullptr;
       const float alpha = p.alpha * (p.alpha_dev ? __ldg(p.alpha_dev) : 1.0f);
-      const float* mrow32 = p.mask32 ? p.mask32 + opix * p.mask32_pitch + p.mask32_coff : nullptr;
       for (int c0 = cpar * 32; c0 < p.block_n; c0 += 64) {
         const bool two = c0 + 16 < p.block_n;
         const int cola = t.n0 + c0, colb = cola + 16;
@@ -125,39 +96,21 @@ __device__ __forceinline__ void epilogue_loop_direct(const UmmaConvParams& p, ui
         tmem_ld16(taddr + c0, ra);
         if (two) tmem_ld16(taddr + c0 + 16, rb);
         tmem_ld_wait();
-        if (valid && cola < p.Cout) store_chunk32(p, alpha, ra, p.bias + cola, orow32 + cola, hrow ? hrow + cola : nullptr, mrow32 ? mrow32 + cola : nullptr, p.out_lo_off);
-        if (two && valid && colb < p.Cout) store_chunk32(p, alpha, rb, p.bias + colb, orow32 + colb, hrow ? hrow + colb : nullptr, mrow32 ? mrow32 + colb : nullptr, p.out_lo_off);
+        if (valid && cola < p.Cout) store_chunk32(p, alpha, ra, p.bias + cola, orow32 + cola, hrow ? hrow + cola : nullptr, nullptr, p.out_lo_off);
+        if (two && valid && colb < p.Cout) store_chunk32(p, alpha, rb, p.bias + colb, orow32 + colb, hrow ? hrow + colb : nullptr, nullptr, p.out_lo_off);
       }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&tempty_bar[acc]);
-      if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      continue;
-    }
-    // two 16-column chunks per iteration: the global loads of both (accumulate / mask operands) and both TMEM
-    // loads are in flight before the first use
-    for (int c0 = cpar * 32; c0 < p.block_n; c0 += 64) {
-      const bool two = c0 + 16 < p.block_n;                       // warp-uniform
-      const int cola = t.n0 + c0, colb = cola + 16;
-      const bool va = valid && cola < p.Cout, vb = two && valid && colb < p.Cout;
-      uint4* da = reinterpret_cast<uint4*>((cola < p.n_split ? orow : orow2) + cola);
-      uint4* db2 = reinterpret_cast<uint4*>((colb < p.n_split ? orow : orow2) + colb);
-      uint4 oa0 = {}, oa1 = {}, ob0 = {}, ob1 = {}, ya0 = {}, ya1 = {}, yb0 = {}, yb1 = {};
-      if (p.accumulate) {
-        if (va) { oa0 = da[0]; oa1 = da[1]; }
-        if (vb) { ob0 = db2[0]; ob1 = db2[1]; }
+    } else {
+      // two 16-column chunks per iteration: both TMEM loads are in flight before the first use
+      for (int c0 = cpar * 32; c0 < p.block_n; c0 += 64) {
+        const bool two = c0 + 16 < p.block_n;                       // warp-uniform
+        const int cola = t.n0 + c0, colb = cola + 16;
+        uint32_t ra[16], rb[16];
+        tmem_ld16(taddr + c0, ra);
+        if (two) tmem_ld16(taddr + c0 + 16, rb);
+        tmem_ld_wait();
+        if (valid && cola < p.Cout) epilogue_chunk(p, ra, cola, reinterpret_cast<uint4*>(orow + cola));
+        if (two && valid && colb < p.Cout) epilogue_chunk(p, rb, colb, reinterpret_cast<uint4*>(orow + colb));
       }
-      if (p.mask_y) {
-        const uint4* my = reinterpret_cast<const uint4*>(p.mask_y + opix * p.mask_pitch + p.mask_coff + cola);
-        if (va) { ya0 = __ldg(my); ya1 = __ldg(my + 1); }
-        if (vb) { yb0 = __ldg(my + 2); yb1 = __ldg(my + 3); }
-      }
-      uint32_t ra[16], rb[16];
-      tmem_ld16(taddr + c0, ra);
-      if (two) tmem_ld16(taddr + c0 + 16, rb);
-      tmem_ld_wait();
-      if (va) epilogue_chunk(p, ra, cola, da, oa0, oa1, ya0, ya1);
-      if (vb) epilogue_chunk(p, rb, colb, db2, ob0, ob1, yb0, yb1);
     }
     tc_fence_before();
     __syncwarp();
@@ -169,9 +122,8 @@ __device__ __forceinline__ void epilogue_loop_direct(const UmmaConvParams& p, ui
 }
 
 __global__ void __launch_bounds__(NUM_THREADS, 1)
-umma_conv_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a2,
-                 const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_a_lo,
-                 const __grid_constant__ CUtensorMap tmap_a2_lo, const __grid_constant__ CUtensorMap tmap_b_lo, const UmmaConvParams p) {
+umma_conv_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                 const __grid_constant__ CUtensorMap tmap_a_lo, const __grid_constant__ CUtensorMap tmap_b_lo, const UmmaConvParams p) {
   extern __shared__ uint8_t smem_raw[];
   // SWIZZLE_128B operand tiles need 1024-byte alignment
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -191,7 +143,6 @@ umma_conv_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_a)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_a2)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_b)) : "memory");
     for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], EPI_WARPS); }
@@ -218,17 +169,14 @@ umma_conv_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
         for (int tap = 0; tap < p.ntaps; ++tap) {
           for (int kc = 0; kc < p.kchunks; ++kc) {
             const CUtensorMap* ma = seg == 0 ? &tmap_a_lo : &tmap_a;
-            const CUtensorMap* ma2 = seg == 0 ? &tmap_a2_lo : &tmap_a2;
             const CUtensorMap* mb = seg == 1 ? &tmap_b_lo : &tmap_b;
             mbar_wait(&empty_bar[stage], phase ^ 1);
             uint8_t* sa = smem + stage * STAGE_BYTES;
             uint8_t* sb = sa + A_BYTES;
-            const uint32_t a_bytes = (uint32_t)(p.bw * p.bh * p.bf) * BLOCK_K * 2;
-            mbar_expect_tx(&full_bar[stage], ((p.ablate & 32) ? 0u : a_bytes) + ((p.ablate & 16) ? 0u : tx_bytes - a_bytes));
-            if (p.ablate & 32) {}
-            else if (kc < p.kchunks_a1) tma_load_4d(sa, ma, &full_bar[stage], kc * BLOCK_K, t.w0 * p.a_stride + p.tap_dx[tap], t.h0 * p.a_stride + p.tap_dy[tap], t.f0);
-            else tma_load_4d(sa, ma2, &full_bar[stage], (kc - p.kchunks_a1) * BLOCK_K, t.w0 + p.tap_dx[tap], t.h0 + p.tap_dy[tap], t.f0);
-            if (!(p.ablate & 16)) tma_load_3d(sb, mb, &full_bar[stage], kc * BLOCK_K, t.n0, tap);
+            mbar_expect_tx(&full_bar[stage], tx_bytes);
+            // output pixel (w0, h0) reads input pixel (2 w0 + dx, 2 h0 + dy); the box steps by 2 (element stride)
+            tma_load_4d(sa, ma, &full_bar[stage], kc * BLOCK_K, 2 * t.w0 + p.tap_dx[tap], 2 * t.h0 + p.tap_dy[tap], t.f0);
+            tma_load_3d(sb, mb, &full_bar[stage], kc * BLOCK_K, t.n0, tap);
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
           }
         }
@@ -250,9 +198,8 @@ umma_conv_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES);
           const uint32_t sb = sa + A_BYTES;
           // K chunks whose tail is TMA zero fill (Cin % 64 != 0) skip the all-zero MMAs
-          const int kvalid = kc < p.kchunks_a1 ? p.K1 - kc * BLOCK_K : p.K - p.K1 - (kc - p.kchunks_a1) * BLOCK_K;
-          if (p.ablate & 8) {
-          } else if (kvalid >= BLOCK_K) {
+          const int kvalid = p.K - kc * BLOCK_K;
+          if (kvalid >= BLOCK_K) {
 #pragma unroll
             for (int k = 0; k < BLOCK_K / UMMA_K; ++k)
               umma_f16(d_tmem, make_desc_k_sw128(sa + k * UMMA_K * 2), make_desc_k_sw128(sb + k * UMMA_K * 2), idesc, (ks | k) ? 1u : 0u);
@@ -271,7 +218,7 @@ umma_conv_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
     }
   } else {
     // ===== epilogue warps 2..9; TMEM lane quadrant = warp % 4, column-group parity = (warp - 2) / 4 =====
-    epilogue_loop_direct(p, tmem_base, tfull_bar, tempty_bar, warp, lane, total_tiles, blockIdx.x, gridDim.x);
+    epilogue_loop(p, tmem_base, tfull_bar, tempty_bar, warp, lane, total_tiles, blockIdx.x, gridDim.x);
   }
 
   tc_fence_before();
@@ -327,139 +274,110 @@ void pick_box(int W, int& bw, int& bh, int& bf) {
   else { bw = 1; bh = 1; bf = 128; }
 }
 
-int bind_common(UmmaContext& ctx, UmmaConvPlan& plan, View a, View o, int F, int K, int N, int ntaps, int out_stride, const __half* w,
-                int a_stride = 1, const UmmaTcOpts* tc = nullptr) {
+// Fields shared by both kernels: the N split, K chunks, output view, weight-map geometry and the SSNB_EXACT_TC epilogue.
+// Tiles enumerate the pixels of the output view `o`; bind_strided or bind_halo then chooses the box, encodes the tensor maps
+// and enables the plan.
+int bind_common(UmmaContext& ctx, UmmaConvPlan& plan, View a, View o, int F, int K, int N, int ntaps, const __half* w,
+                const UmmaTcOpts* tc) {
   plan.enabled = false;
   if (int rc = resolve_encode(ctx)) return rc;
-  if (a_stride == 2) {
-    // strided TMA: tiles enumerate OUTPUT pixels, the A box steps over the input with stride 2
-    View ao = a; ao.H = o.H; ao.W = o.W;
-    if (int rc = bind_common(ctx, plan, ao, o, F, K, N, ntaps, 1, w, 1, tc)) return rc;
-    plan.enabled = false;
-    UmmaConvParams& q = plan.p;
-    q.a_stride = 2;
-    cuuint64_t dims[4] = {(cuuint64_t)K, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)F};
-    cuuint64_t str[3] = {(cuuint64_t)a.pitch * 2, (cuuint64_t)a.W * a.pitch * 2, (cuuint64_t)a.H * a.W * a.pitch * 2};
-    cuuint32_t box[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)(2 * q.bw), (cuuint32_t)(2 * q.bh), (cuuint32_t)q.bf};
-    if (int rc = encode(ctx, &plan.tmap_a, 4, reinterpret_cast<__half*>(a.base) + a.coff, dims, str, box, 2)) return rc;
-    plan.tmap_a_lo = plan.tmap_a;
-    if (a.lo_off)
-      if (int rc = encode(ctx, &plan.tmap_a_lo, 4, reinterpret_cast<__half*>(reinterpret_cast<char*>(a.base) + a.lo_off) + a.coff, dims, str, box, 2)) return rc;
-    plan.tmap_a2 = plan.tmap_a; plan.tmap_a2_lo = plan.tmap_a_lo;
-    plan.enabled = true;
-    return 0;
-  }
-  if ((a.H + out_stride - 1) / out_stride != o.H || (a.W + out_stride - 1) / out_stride != o.W) { set_thread_error("umma conv: geometry mismatch"); return 1; }
   if (K % 8 || N % 16 || a.pitch % 8 || a.coff % 8 || o.pitch % 8 || o.coff % 8 || ntaps > UMMA_MAX_TAPS) {
     set_thread_error("umma conv: unsupported channel alignment"); return 1; }
   UmmaConvParams& p = plan.p;
   memset(&p, 0, sizeof(p));
-  p.W = a.W; p.H = a.H; p.F = F;
-  pick_box(a.W, p.bw, p.bh, p.bf);
-  p.tiles_w = (a.W + p.bw - 1) / p.bw; p.tiles_h = (a.H + p.bh - 1) / p.bh; p.tiles_f = (F + p.bf - 1) / p.bf;
+  p.W = o.W; p.H = o.H; p.F = F;
   // N split: equal tiles of block_n <= 256 (multiple of 16); the last tile may overhang N (TMA zero-fills the
   // missing weight rows, the epilogue masks the columns)
   p.n_tiles = (N + 255) / 256;
   p.block_n = (((N + p.n_tiles - 1) / p.n_tiles) + 15) / 16 * 16;
   p.kchunks = (K + BLOCK_K - 1) / BLOCK_K;
   p.K = K;
-  p.stage_bytes = (A_BYTES + p.block_n * BLOCK_K * 2 + 1023) / 1024 * 1024;
-  p.stages = PIPE_BYTES / p.stage_bytes; if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
   p.ntaps = ntaps;
   p.out = reinterpret_cast<__half*>(o.base); p.out_pitch = o.pitch; p.out_coff = o.coff; p.Cout = N;
-  p.out_stride = out_stride; p.OH = o.H; p.OW = o.W; p.a_stride = 1; p.mask_y = nullptr; p.mask_pitch = 0; p.mask_coff = 0;
-  p.kchunks_a1 = (K + BLOCK_K - 1) / BLOCK_K; p.K1 = K; p.n_split = 1 << 30; p.out2 = p.out; p.out2_pitch = o.pitch; p.out2_coff = o.coff;
-  {
-    cuuint64_t dims[4] = {(cuuint64_t)K, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)F};
-    cuuint64_t str[3] = {(cuuint64_t)a.pitch * 2, (cuuint64_t)a.W * a.pitch * 2, (cuuint64_t)a.H * a.W * a.pitch * 2};
-    cuuint32_t box[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)p.bw, (cuuint32_t)p.bh, (cuuint32_t)p.bf};
-    if (int rc = encode(ctx, &plan.tmap_a, 4, reinterpret_cast<__half*>(a.base) + a.coff, dims, str, box)) return rc;
-    plan.tmap_a_lo = plan.tmap_a;
-    if (a.lo_off)
-      if (int rc = encode(ctx, &plan.tmap_a_lo, 4, reinterpret_cast<__half*>(reinterpret_cast<char*>(a.base) + a.lo_off) + a.coff, dims, str, box)) return rc;
-  }
-  {
-    cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)N, (cuuint64_t)ntaps};
-    cuuint64_t str[2] = {(cuuint64_t)K * 2, (cuuint64_t)N * K * 2};
-    cuuint32_t box[3] = {(cuuint32_t)BLOCK_K, (cuuint32_t)p.block_n, 1};
-    if (int rc = encode(ctx, &plan.tmap_b, 3, const_cast<__half*>(w), dims, str, box)) return rc;
-    plan.b_ptr = w;
-    plan.b_lo_off = tc ? tc->w_lo_off : 0;
-    plan.tmap_b_lo = plan.tmap_b;
-    if (plan.b_lo_off)
-      if (int rc = encode(ctx, &plan.tmap_b_lo, 3, reinterpret_cast<__half*>(reinterpret_cast<char*>(const_cast<__half*>(w)) + plan.b_lo_off), dims, str, box)) return rc;
-    for (int i = 0; i < 3; ++i) plan.b_dims[i] = dims[i];
-    for (int i = 0; i < 2; ++i) plan.b_strides[i] = str[i];
-  }
-  plan.tmap_a2 = plan.tmap_a; plan.tmap_a2_lo = plan.tmap_a_lo;
+  p.kchunks_a1 = p.kchunks; p.K1 = K; p.n_split = 1 << 30; p.out2 = p.out; p.out2_pitch = o.pitch; p.out2_coff = o.coff;
+  plan.b_ptr = w;
+  plan.b_lo_off = tc ? tc->w_lo_off : 0;
+  plan.b_dims[0] = K; plan.b_dims[1] = N; plan.b_dims[2] = ntaps;
+  plan.b_strides[0] = (unsigned long long)K * 2; plan.b_strides[1] = (unsigned long long)N * K * 2;
   // SSNB_EXACT_TC: three operand segments per K chunk, fp32 epilogue (+ fp16 operand planes of the result)
   p.nseg = tc ? 3 : 1; p.out_f32 = tc ? 1 : 0; p.alpha = tc ? tc->alpha : 1.0f; p.alpha_dev = tc ? tc->alpha_dev : nullptr;
-  p.mask32 = nullptr; p.mask32_pitch = 0; p.mask32_coff = 0; p.plane_scale = 1.0f; p.flag = nullptr;
+  p.plane_scale = 1.0f;
   p.out32 = tc ? tc->out32 : nullptr; p.out_hi = tc ? reinterpret_cast<__half*>(o.base) : nullptr; p.out_lo_off = tc ? o.lo_off : 0;
   p.out32_2 = p.out32; p.out_hi2 = p.out_hi; p.out_lo_off2 = p.out_lo_off;       // second destination = the first unless a fused bind redirects it
   if (tc && (!tc->out32 || !a.lo_off || !tc->w_lo_off)) { set_thread_error("umma conv: split-operand bind needs operand planes and an fp32 output"); return 1; }
+  return 0;
+}
+
+// weight map (and its LO plane) with boxes of BLOCK_K channels x `rows` output channels x `taps` taps
+int encode_b(UmmaContext& ctx, UmmaConvPlan& plan, int rows, int taps) {
+  cuuint64_t dims[3] = {plan.b_dims[0], plan.b_dims[1], plan.b_dims[2]};
+  cuuint64_t str[2] = {plan.b_strides[0], plan.b_strides[1]};
+  cuuint32_t box[3] = {(cuuint32_t)BLOCK_K, (cuuint32_t)rows, (cuuint32_t)taps};
+  __half* w = const_cast<__half*>(plan.b_ptr);
+  if (int rc = encode(ctx, &plan.tmap_b, 3, w, dims, str, box)) return rc;
+  plan.tmap_b_lo = plan.tmap_b;
+  if (plan.b_lo_off) return encode(ctx, &plan.tmap_b_lo, 3, reinterpret_cast<__half*>(reinterpret_cast<char*>(w) + plan.b_lo_off), dims, str, box);
+  return 0;
+}
+
+// Stride-2 forward on the first-generation kernel: tiles enumerate OUTPUT pixels, the A box steps over the input `a` with
+// TMA element stride 2 (box extents in un-strided elements).
+int bind_strided(UmmaContext& ctx, UmmaConvPlan& plan, View a) {
+  UmmaConvParams& p = plan.p;
+  pick_box(p.W, p.bw, p.bh, p.bf);
+  p.tiles_w = (p.W + p.bw - 1) / p.bw; p.tiles_h = (p.H + p.bh - 1) / p.bh; p.tiles_f = (p.F + p.bf - 1) / p.bf;
+  p.stage_bytes = (A_BYTES + p.block_n * BLOCK_K * 2 + 1023) / 1024 * 1024;
+  p.stages = PIPE_BYTES / p.stage_bytes; if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
+  cuuint64_t dims[4] = {(cuuint64_t)p.K, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)p.F};
+  cuuint64_t str[3] = {(cuuint64_t)a.pitch * 2, (cuuint64_t)a.W * a.pitch * 2, (cuuint64_t)a.H * a.W * a.pitch * 2};
+  cuuint32_t box[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)(2 * p.bw), (cuuint32_t)(2 * p.bh), (cuuint32_t)p.bf};
+  if (int rc = encode(ctx, &plan.tmap_a, 4, reinterpret_cast<__half*>(a.base) + a.coff, dims, str, box, 2)) return rc;
+  plan.tmap_a_lo = plan.tmap_a;
+  if (a.lo_off)
+    if (int rc = encode(ctx, &plan.tmap_a_lo, 4, reinterpret_cast<__half*>(reinterpret_cast<char*>(a.base) + a.lo_off) + a.coff, dims, str, box, 2)) return rc;
+  if (int rc = encode_b(ctx, plan, p.block_n, 1)) return rc;
   plan.enabled = true;
   return 0;
 }
 
-// Route a bound stride-1 plan to the second-generation kernel (umma_conv_v2.cu): halo layout (one A box per K chunk
-// covers the tile plus the filter border, taps = shifted UMMA descriptor views; a 1x1 layer is the halo-free case),
-// several taps per weight stage, CTA pairs.
-//   SSNB_V2=0            keep every layer on the first-generation kernel of this file
-//   SSNB_PAIR=0          single-CTA MMAs (cta_group::1) instead of CTA pairs
-//   SSNB_HALO_MODE=m     how horizontal shifts are realised: 2 (default) halo rows at their exact pitch (bw + halo pixels);
-//                        1 rows padded to a 16-pixel pitch; 4 one box per horizontal shift (every view 1024-byte aligned).
-//                        Measured on B200 (tools/halo_probe.sh): the UMMA unit applies the 128-byte swizzle to absolute
-//                        shared-memory address bits, so views that start at any 128-byte row of a TMA-written tile read
-//                        correctly with descriptor base_offset 0 (a non-zero base_offset gives wrong data).
-//   SSNB_HALO_MIN_W=w    smallest image width that uses it (default 7: every stride-1 layer)
+// Stride-1 plans run on the second-generation kernel (umma_conv_v2.cu): halo layout (one A box per K chunk covers the
+// tile plus the filter border, taps = shifted UMMA descriptor views; a 1x1 layer is the halo-free case), several taps per
+// weight stage, CTA pairs.  A halo row holds its pixels at their exact pitch (bw + halo pixels).  Measured on B200: the
+// UMMA unit applies the 128-byte swizzle to absolute shared-memory address bits, so views that start at any 128-byte row
+// of a TMA-written tile read correctly with descriptor base_offset 0 (a non-zero base_offset gives wrong data).
+// A plan that this kernel cannot take fails the bind.
 // `a2` is the second activation source of a fused sibling data gradient (K chunks >= kchunks_a1), or nullptr.
 constexpr int V2_STAGES_MAX = 8;
-int try_halo(UmmaContext& ctx, UmmaConvPlan& plan, View a, int F, const View* a2 = nullptr) {
+int bind_halo(UmmaContext& ctx, UmmaConvPlan& plan, View a, int F, const View* a2 = nullptr) {
   UmmaConvParams& p = plan.p;
-  p.halo = 0; p.pair = 0; p.v2 = 0;
-  const char* ve = getenv("SSNB_V2");
-  if ((ve && ve[0] == '0') || !umma_conv_v2_supported(p.ntaps)) return 0;
-  const char* pe = getenv("SSNB_PAIR");
-  const bool pair = !(pe && pe[0] == '0');
-  if (!plan.enabled || p.a_stride != 1 || p.out_stride != 1) return 0;
-  if (p.kchunks_a1 != p.kchunks && (p.ntaps != 1 || !a2)) return 0;
+  auto fail = [](const char* why) { set_thread_error(std::string("umma conv v2: ") + why); return 1; };
+  if (a.H != p.H || a.W != p.W) return fail("geometry mismatch");
+  if (!umma_conv_v2_supported(p.ntaps)) return fail("no kernel instance for this tap count");
   // the v2 epilogue moves 16 fp16 columns per 256-bit access: rows and channel slices must be 32-byte aligned; its
   // shared-memory bias table holds 1024 columns
-  if (p.out_pitch % 16 || p.out_coff % 16 || p.out2_pitch % 16 || p.out2_coff % 16 || p.n_split % 16 || (p.bias && p.n_tiles * p.block_n > 1024)) return 0;
-  if (plan.mask_y && (plan.mask_pitch % 16 || plan.mask_coff % 16)) return 0;
-  const char* mw = getenv("SSNB_HALO_MIN_W");
-  if (a.W < (mw ? atoi(mw) : 7)) return 0;
-  const char* md = getenv("SSNB_HALO_MODE");
-  const int mode = md ? atoi(md) : 2;
+  if (p.out_pitch % 16 || p.out_coff % 16 || p.out2_pitch % 16 || p.out2_coff % 16 || p.n_split % 16) return fail("output views are not 32-byte aligned");
+  if (p.bias && p.n_tiles * p.block_n > 1024) return fail("more than 1024 bias columns");
   int x0 = 0, x1 = 0, y0 = 0, y1 = 0;
   for (int t = 0; t < p.ntaps; ++t) {
     x0 = std::min(x0, p.tap_dx[t]); x1 = std::max(x1, p.tap_dx[t]);
     y0 = std::min(y0, p.tap_dy[t]); y1 = std::max(y1, p.tap_dy[t]);
   }
-  const int xh = x1 - x0, yh = y1 - y0;
   int bh = 8;
   while (bh > 1 && a.H % bh) bh >>= 1;
   const int bw = 8, bf = BLOCK_M / (bw * bh);
-  int loads = 1, pw;
-  if (xh == 0) pw = bw;
-  else if (mode == 4) { loads = xh + 1; pw = bw; }
-  else if (mode >= 2) pw = bw + xh;
-  else pw = 16;
-  const int bhh = bh + yh;
-  if (loads > 4 || bhh > 256 || bf > 256) return 0;
-  // TMA-fed epilogue for data gradients (default; SSNB_EPI_TMA=0 keeps the register-prefetch epilogue -- measured on B200,
-  // round 2: 9.82 vs 10.00 ms per training step, 0 mismatching launches in tools/umma_diag.py): a ring of 3 x (old-gradient + activation chunk) at the
-  // top of the staging area; the operand rings get what is left
-  const char* te = getenv("SSNB_EPI_TMA");
-  const bool want_ring = !(te && te[0] == '0') && !p.bias && !p.relu && !p.out_f32;
+  const int pw = bw + (x1 - x0), bhh = bh + (y1 - y0);
+  if (bhh > 256 || bf > 256) return fail("box limits");
+  // TMA-fed epilogue for data gradients (measured on B200, round 2: 9.82 vs 10.00 ms per training step against the
+  // register-prefetch epilogue, 0 mismatching launches in tools/umma_diag.py): a ring of 3 x (old-gradient + activation
+  // chunk) at the top of the staging area; the operand rings get what is left
+  const bool want_ring = !p.bias && !p.relu && !p.out_f32;
   constexpr int EPI_STAGE = 2 * 128 * 128, EPI_STAGES = 3;
   int pipe = UMMA_V2_PIPE_BYTES - (want_ring ? EPI_STAGES * EPI_STAGE : 0);
   bool ring = want_ring;
 retry_without_ring:
-  const int b_rows = pair ? p.block_n / 2 : p.block_n;      // weight rows each CTA stages per (tap, K chunk)
+  const int b_rows = p.block_n / 2;                         // weight rows each CTA of the pair stages per (tap, K chunk)
   const int a_load_bytes = pw * bf * bhh * BLOCK_K * 2;
-  const int a_stage = (loads * a_load_bytes + 1023) / 1024 * 1024;
+  const int a_stage = (a_load_bytes + 1023) / 1024 * 1024;
   const int slab = b_rows * BLOCK_K * 2;                    // one tap of the weight stage (multiple of 1024: rows % 8 == 0)
   int b_taps = 1;
   if (p.ntaps > 1) {                                        // several taps per weight stage: fewer barrier hand-offs per K chunk
@@ -470,27 +388,21 @@ retry_without_ring:
   int a_stages, b_stages;
   if (p.ntaps == 1) {                                       // one box + one slab per step: equal ring depths
     a_stages = b_stages = std::min(V2_STAGES_MAX, pipe / (a_stage + b_stage));
-    if (a_stages < 3) { if (ring) { ring = false; pipe = UMMA_V2_PIPE_BYTES; goto retry_without_ring; } return 0; }
+    if (a_stages < 3) { if (ring) { ring = false; pipe = UMMA_V2_PIPE_BYTES; goto retry_without_ring; } return fail("operand stages do not fit"); }
   } else {
     a_stages = 3;
     if ((pipe - 3 * a_stage) / b_stage < 3) a_stages = 2;
     b_stages = (pipe - a_stages * a_stage) / b_stage;
-    if (b_stages < 2) { if (ring) { ring = false; pipe = UMMA_V2_PIPE_BYTES; goto retry_without_ring; } return 0; }   // does not fit: stay on the first-generation kernel
+    if (b_stages < 2) { if (ring) { ring = false; pipe = UMMA_V2_PIPE_BYTES; goto retry_without_ring; } return fail("operand stages do not fit"); }
     if (b_stages > V2_STAGES_MAX) b_stages = V2_STAGES_MAX;
   }
   p.v2 = 1; p.b_taps = b_taps;
-  p.halo = 1; p.pair = pair ? 1 : 0;
   p.bw = bw; p.bh = bh; p.bf = bf;
   p.tiles_w = (a.W + bw - 1) / bw; p.tiles_h = (a.H + bh - 1) / bh; p.tiles_f = (F + bf - 1) / bf;
-  p.tiles_q = pair ? (p.tiles_f + 1) / 2 : p.tiles_f;
+  p.tiles_q = (p.tiles_f + 1) / 2;
   p.a_stages = a_stages; p.b_stages = b_stages; p.a_stage_bytes = a_stage; p.b_stage_bytes = b_stage;
-  p.a_loads = loads; p.a_load_bytes = a_load_bytes; p.halo_x0 = x0; p.halo_y0 = y0; p.a_sbo = pw * BLOCK_K * 2;
-  for (int l = 0; l < 4; ++l) p.a_load_dx[l] = loads > 1 ? l : 0;
-  for (int t = 0; t < p.ntaps; ++t) {
-    const int l = loads > 1 ? p.tap_dx[t] - x0 : 0;
-    const int dxl = loads > 1 ? 0 : p.tap_dx[t] - x0;
-    p.tap_aoff[t] = l * a_load_bytes + ((p.tap_dy[t] - y0) * bf * pw + dxl) * BLOCK_K * 2;
-  }
+  p.a_load_bytes = a_load_bytes; p.halo_x0 = x0; p.halo_y0 = y0; p.a_sbo = pw * BLOCK_K * 2;
+  for (int t = 0; t < p.ntaps; ++t) p.tap_aoff[t] = ((p.tap_dy[t] - y0) * bf * pw + p.tap_dx[t] - x0) * BLOCK_K * 2;
   // halo box: dims {C, W, F, H} so that shared memory holds [y][frame][x][64 ch]
   auto encode_a = [&](CUtensorMap* m, const View& v, int channels) -> int {
     cuuint64_t dims[4] = {(cuuint64_t)channels, (cuuint64_t)v.W, (cuuint64_t)F, (cuuint64_t)v.H};
@@ -499,37 +411,29 @@ retry_without_ring:
     return encode(ctx, m, 4, reinterpret_cast<__half*>(v.base) + v.coff, dims, str, box);
   };
   auto lo_of = [](View v) { v.base = reinterpret_cast<char*>(v.base) + v.lo_off; return v; };
-  if (int rc = encode_a(&plan.tmap_a, a, p.K1)) { plan.enabled = false; return rc; }
+  if (int rc = encode_a(&plan.tmap_a, a, p.K1)) return rc;
   plan.tmap_a_lo = plan.tmap_a;
-  if (a.lo_off) if (int rc = encode_a(&plan.tmap_a_lo, lo_of(a), p.K1)) { plan.enabled = false; return rc; }
-  if (p.kchunks_a1 != p.kchunks) {
-    if (int rc = encode_a(&plan.tmap_a2, *a2, p.K - p.K1)) { plan.enabled = false; return rc; }
+  if (a.lo_off) if (int rc = encode_a(&plan.tmap_a_lo, lo_of(a), p.K1)) return rc;
+  if (a2) {
+    if (int rc = encode_a(&plan.tmap_a2, *a2, p.K - p.K1)) return rc;
     plan.tmap_a2_lo = plan.tmap_a2;
-    if (a2->lo_off) if (int rc = encode_a(&plan.tmap_a2_lo, lo_of(*a2), p.K - p.K1)) { plan.enabled = false; return rc; }
+    if (a2->lo_off) if (int rc = encode_a(&plan.tmap_a2_lo, lo_of(*a2), p.K - p.K1)) return rc;
   } else { plan.tmap_a2 = plan.tmap_a; plan.tmap_a2_lo = plan.tmap_a_lo; }
   p.epi_stages = 0; p.epi_stage_bytes = 0; plan.epi_maps_ready = false; plan.epi_mask_ready = false;
   if (ring) {                                               // TMA-fed epilogue: [128 rows][64 ch] boxes of the output view
     p.epi_stages = EPI_STAGES; p.epi_stage_bytes = EPI_STAGE;
     plan.epi_box[0] = bw; plan.epi_box[1] = bf; plan.epi_box[2] = bh; plan.epi_F = F;
-    cuuint64_t od[4] = {(cuuint64_t)p.Cout, (cuuint64_t)p.OW, (cuuint64_t)F, (cuuint64_t)p.OH};
-    cuuint64_t os[3] = {(cuuint64_t)p.out_pitch * 2, (cuuint64_t)p.OH * p.OW * p.out_pitch * 2, (cuuint64_t)p.OW * p.out_pitch * 2};
+    cuuint64_t od[4] = {(cuuint64_t)p.Cout, (cuuint64_t)p.W, (cuuint64_t)F, (cuuint64_t)p.H};
+    cuuint64_t os[3] = {(cuuint64_t)p.out_pitch * 2, (cuuint64_t)p.H * p.W * p.out_pitch * 2, (cuuint64_t)p.W * p.out_pitch * 2};
     cuuint32_t ob[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)bw, (cuuint32_t)bf, (cuuint32_t)bh};
-    if (int rc = encode(ctx, &plan.tmap_old, 4, p.out + p.out_coff, od, os, ob)) { plan.enabled = false; return rc; }
+    if (int rc = encode(ctx, &plan.tmap_old, 4, p.out + p.out_coff, od, os, ob)) return rc;
     plan.tmap_y = plan.tmap_old;
     plan.epi_maps_ready = true;
   } else {
     plan.tmap_old = plan.tmap_a; plan.tmap_y = plan.tmap_a;  // valid descriptors, never dereferenced
   }
-  if (pair || b_taps > 1) {                                 // pair: each CTA stages half of the weight rows; v2: b_taps taps per stage
-    cuuint64_t bd[3] = {plan.b_dims[0], plan.b_dims[1], plan.b_dims[2]};
-    cuuint64_t bs[2] = {plan.b_strides[0], plan.b_strides[1]};
-    cuuint32_t bb[3] = {(cuuint32_t)BLOCK_K, (cuuint32_t)b_rows, (cuuint32_t)b_taps};
-    if (int rc = encode(ctx, &plan.tmap_b, 3, const_cast<__half*>(plan.b_ptr), bd, bs, bb)) { plan.enabled = false; return rc; }
-    plan.tmap_b_lo = plan.tmap_b;
-    if (plan.b_lo_off)
-      if (int rc = encode(ctx, &plan.tmap_b_lo, 3, reinterpret_cast<__half*>(reinterpret_cast<char*>(const_cast<__half*>(plan.b_ptr)) + plan.b_lo_off), bd, bs, bb)) {
-        plan.enabled = false; return rc; }
-  }
+  if (int rc = encode_b(ctx, plan, b_rows, b_taps)) return rc;
+  plan.enabled = true;
   return 0;
 }
 
@@ -546,34 +450,29 @@ void umma_context_destroy(UmmaContext&) {}
 
 int umma_conv_bind_taps(UmmaContext& ctx, UmmaConvPlan& plan, View in, View out, int F, int cin, int cout, int ntaps,
                         const int* dy, const int* dx, const __half* w_tap_n_k, const float* bias, int relu, const UmmaTcOpts* tc) {
-  if (int rc = bind_common(ctx, plan, in, out, F, cin, cout, ntaps, 1, w_tap_n_k, 1, tc)) return rc;
+  if (int rc = bind_common(ctx, plan, in, out, F, cin, cout, ntaps, w_tap_n_k, tc)) return rc;
   for (int t = 0; t < ntaps; ++t) { plan.p.tap_dy[t] = dy[t]; plan.p.tap_dx[t] = dx[t]; }
   plan.p.bias = bias; plan.p.relu = relu; plan.p.accumulate = 0;
-  return try_halo(ctx, plan, in, F);
+  return bind_halo(ctx, plan, in, F);
 }
 
 int umma_conv_bind_fwd(UmmaContext& ctx, UmmaConvPlan& plan, View in, View out, int F, int cin, int cout, int k, int pad,
                        int stride, const __half* w_tap_n_k, const float* bias, const UmmaTcOpts* tc) {
-  // a stride-2 layer (k=3, pad=1): tiles over OUTPUT pixels whose A boxes step over the input with TMA element
-  // stride 2 (default), or the stride-1 convolution sampled at even pixels (4x redundant MMAs, SSNB_TMA_STRIDED=0)
-  const char* st = getenv("SSNB_TMA_STRIDED");           // default on; "0" falls back to the sampled-epilogue variant
-  const bool strided = stride == 2 && !(st && st[0] == '0');
-  if (int rc = strided ? bind_common(ctx, plan, in, out, F, cin, cout, k * k, 1, w_tap_n_k, 2, tc)
-                       : bind_common(ctx, plan, in, out, F, cin, cout, k * k, stride, w_tap_n_k, 1, tc)) return rc;
+  if (int rc = bind_common(ctx, plan, in, out, F, cin, cout, k * k, w_tap_n_k, tc)) return rc;
   for (int r = 0; r < k; ++r)
     for (int s = 0; s < k; ++s) { plan.p.tap_dy[r * k + s] = r - pad; plan.p.tap_dx[r * k + s] = s - pad; }
   plan.p.bias = bias; plan.p.relu = 1; plan.p.accumulate = 0;
-  return try_halo(ctx, plan, in, F);
+  return stride == 2 ? bind_strided(ctx, plan, in) : bind_halo(ctx, plan, in, F);
 }
 
 int umma_conv_bind_dgrad(UmmaContext& ctx, UmmaConvPlan& plan, View dz, View dx, int F, int cin, int cout, int k, int pad,
                          const __half* w_tap_k_n, int accumulate, const UmmaTcOpts* tc) {
   // dx[p, ci] = sum_{r,s,co} dz[p + (pad-r, pad-s), co] * W[co][ci][r][s] : K = cout, N = cin
-  if (int rc = bind_common(ctx, plan, dz, dx, F, cout, cin, k * k, 1, w_tap_k_n, 1, tc)) return rc;
+  if (int rc = bind_common(ctx, plan, dz, dx, F, cout, cin, k * k, w_tap_k_n, tc)) return rc;
   for (int r = 0; r < k; ++r)
     for (int s = 0; s < k; ++s) { plan.p.tap_dy[r * k + s] = pad - r; plan.p.tap_dx[r * k + s] = pad - s; }
   plan.p.bias = nullptr; plan.p.relu = 0; plan.p.accumulate = accumulate;
-  return try_halo(ctx, plan, dz, F);
+  return bind_halo(ctx, plan, dz, F);
 }
 
 int umma_conv_bind_fused_fwd(UmmaContext& ctx, UmmaConvPlan& plan, View in, View out1, View out2, int F, int cin, int n1, int n2,
@@ -581,7 +480,7 @@ int umma_conv_bind_fused_fwd(UmmaContext& ctx, UmmaConvPlan& plan, View in, View
   // bind as one convolution with N = n1 + n2 writing to out1's geometry, then redirect columns >= n1
   View o = out1; o.C = n1 + n2;
   if (out1.H != out2.H || out1.W != out2.W || n1 % 16 || n2 % 16 || out2.pitch % 8 || out2.coff % 8) { set_thread_error("fused fwd: bad views"); return 1; }
-  if (int rc = bind_common(ctx, plan, in, o, F, cin, n1 + n2, 1, 1, w_n_k, 1, tc)) return rc;
+  if (int rc = bind_common(ctx, plan, in, o, F, cin, n1 + n2, 1, w_n_k, tc)) return rc;
   plan.p.tap_dy[0] = 0; plan.p.tap_dx[0] = 0;
   plan.p.bias = bias; plan.p.relu = 1; plan.p.accumulate = 0;
   plan.p.n_split = n1; plan.p.out2 = reinterpret_cast<__half*>(out2.base); plan.p.out2_pitch = out2.pitch; plan.p.out2_coff = out2.coff;
@@ -589,43 +488,32 @@ int umma_conv_bind_fused_fwd(UmmaContext& ctx, UmmaConvPlan& plan, View in, View
     if (!tc->out32_2) { set_thread_error("fused fwd: the split-operand bind needs both fp32 destinations"); return 1; }
     plan.p.out32_2 = tc->out32_2; plan.p.out_hi2 = reinterpret_cast<__half*>(out2.base); plan.p.out_lo_off2 = out2.lo_off;
   }
-  return try_halo(ctx, plan, in, F);
+  return bind_halo(ctx, plan, in, F);
 }
 
 int umma_conv_bind_fused_dgrad(UmmaContext& ctx, UmmaConvPlan& plan, View dz1, View dz2, View dx, int F, int cin, int k1, int k2,
                                const __half* w_n_k, int accumulate, const UmmaTcOpts* tc) {
   const int k1p = (k1 + BLOCK_K - 1) / BLOCK_K * BLOCK_K;
-  // bind with the first source as the A view and the full fused K; then attach the second source
+  // bind with the first source as the A view; then attach the second source and the full fused K
   View a = k1 ? dz1 : dz2;
-  if (int rc = bind_common(ctx, plan, a, dx, F, k1 ? k1 : k2, cin, 1, 1, w_n_k, 1, tc)) return rc;
+  if (int rc = bind_common(ctx, plan, a, dx, F, k1 ? k1 : k2, cin, 1, w_n_k, tc)) return rc;
   UmmaConvParams& p = plan.p;
   p.tap_dy[0] = 0; p.tap_dx[0] = 0; p.bias = nullptr; p.relu = 0; p.accumulate = accumulate;
   if (k1) {
     if (dz2.H != dz1.H || dz2.W != dz1.W || dz2.pitch % 8 || dz2.coff % 8 || k2 % 8) { set_thread_error("fused dgrad: bad views"); return 1; }
-    cuuint64_t dims[4] = {(cuuint64_t)k2, (cuuint64_t)dz2.W, (cuuint64_t)dz2.H, (cuuint64_t)F};
-    cuuint64_t str[3] = {(cuuint64_t)dz2.pitch * 2, (cuuint64_t)dz2.W * dz2.pitch * 2, (cuuint64_t)dz2.H * dz2.W * dz2.pitch * 2};
-    cuuint32_t box[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)p.bw, (cuuint32_t)p.bh, (cuuint32_t)p.bf};
-    if (int rc = encode(ctx, &plan.tmap_a2, 4, reinterpret_cast<__half*>(dz2.base) + dz2.coff, dims, str, box)) { plan.enabled = false; return rc; }
+    if (tc && !dz2.lo_off) { set_thread_error("fused dgrad: the split-operand bind needs the second source's operand planes"); return 1; }
     p.kchunks_a1 = k1p / BLOCK_K; p.K1 = k1; p.K = k1 + k2;
     p.kchunks = p.kchunks_a1 + (k2 + BLOCK_K - 1) / BLOCK_K;
     // the weight map covers the padded fused K
-    cuuint64_t bd[3] = {(cuuint64_t)(k1p + k2), (cuuint64_t)cin, 1};
-    cuuint64_t bs[2] = {(cuuint64_t)(k1p + k2) * 2, (cuuint64_t)cin * (k1p + k2) * 2};
-    cuuint32_t bb[3] = {(cuuint32_t)BLOCK_K, (cuuint32_t)p.block_n, 1};
-    if (int rc = encode(ctx, &plan.tmap_b, 3, const_cast<__half*>(w_n_k), bd, bs, bb)) { plan.enabled = false; return rc; }
-    plan.b_ptr = w_n_k;
-    plan.tmap_b_lo = plan.tmap_b;
-    if (plan.b_lo_off)
-      if (int rc = encode(ctx, &plan.tmap_b_lo, 3, reinterpret_cast<__half*>(reinterpret_cast<char*>(const_cast<__half*>(w_n_k)) + plan.b_lo_off), bd, bs, bb)) {
-        plan.enabled = false; return rc; }
-    for (int i = 0; i < 3; ++i) plan.b_dims[i] = bd[i];
-    for (int i = 0; i < 2; ++i) plan.b_strides[i] = bs[i];
-    if (tc && !dz2.lo_off) { set_thread_error("fused dgrad: the split-operand bind needs the second source's operand planes"); plan.enabled = false; return 1; }
+    plan.b_dims[0] = k1p + k2; plan.b_dims[1] = cin; plan.b_dims[2] = 1;
+    plan.b_strides[0] = (unsigned long long)(k1p + k2) * 2; plan.b_strides[1] = (unsigned long long)cin * (k1p + k2) * 2;
   }
-  return try_halo(ctx, plan, a, F, k1 ? &dz2 : nullptr);
+  return bind_halo(ctx, plan, a, F, k1 ? &dz2 : nullptr);
 }
 
-void umma_conv_set_mask(UmmaContext& ctx, UmmaConvPlan& plan, View y) {
+int umma_conv_set_mask(UmmaContext& ctx, UmmaConvPlan& plan, View y) {
+  // the v2 epilogue reads the activation with 256-bit loads
+  if (y.pitch % 16 || y.coff % 16) { set_thread_error("umma conv: the mask activation view is not 32-byte aligned"); return 1; }
   plan.mask_y = reinterpret_cast<const __half*>(y.base); plan.mask_pitch = y.pitch; plan.mask_coff = y.coff;
   plan.epi_mask_ready = false;
   if (plan.epi_maps_ready) {                                 // TMA-fed epilogue: the activation tiles come through TMA too
@@ -634,6 +522,7 @@ void umma_conv_set_mask(UmmaContext& ctx, UmmaConvPlan& plan, View y) {
     cuuint32_t b[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)plan.epi_box[0], (cuuint32_t)plan.epi_box[1], (cuuint32_t)plan.epi_box[2]};
     plan.epi_mask_ready = encode(ctx, &plan.tmap_y, 4, reinterpret_cast<__half*>(y.base) + y.coff, d, st, b) == 0;
   }
+  return 0;
 }
 
 void umma_conv_set_mask_tc(UmmaConvPlan& plan, View y32, View dplanes, float plane_scale, int* flag) {
@@ -644,24 +533,22 @@ void umma_conv_set_mask_tc(UmmaConvPlan& plan, View y32, View dplanes, float pla
 
 int umma_conv_launch(UmmaContext& ctx, const UmmaConvPlan& plan, cudaStream_t s, bool mask) {
   if (!plan.enabled) { set_thread_error("umma conv: plan not bound"); return 3; }
-  if (!ctx.attr_set) {
-    if (cudaFuncSetAttribute(umma_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess) {
-      set_thread_error("umma conv: cannot raise dynamic shared memory limit"); cudaGetLastError(); return 2; }
-    ctx.attr_set = true;
-  }
   UmmaConvParams p = plan.p;
   if (mask && plan.mask_y) { p.mask_y = plan.mask_y; p.mask_pitch = plan.mask_pitch; p.mask_coff = plan.mask_coff; }
   if (mask && p.out_f32 && plan.mask32) {
     p.mask32 = plan.mask32; p.mask32_pitch = plan.mask32_pitch; p.mask32_coff = plan.mask32_coff;
     p.out_hi = plan.mask_planes; p.out_lo_off = plan.mask_planes_lo; p.plane_scale = plan.mask_plane_scale; p.flag = plan.mask_flag;
   }
-  static const int ablate = [] { const char* e = getenv("SSNB_ABLATE"); return e ? atoi(e) : 0; }();     // timing experiments only
-  p.ablate = ablate;
   if (p.v2) return umma_conv_v2_launch(ctx, plan, p, s);
-  if (p.out_f32 && (p.mask_y || p.n_split < p.Cout || p.out_stride != 1)) { set_thread_error("umma conv: the fp32 epilogue has no mask / second destination / sampling"); return 3; }
+  // stride-2 forward: the first-generation kernel of this file
+  if (!ctx.attr_set) {
+    if (cudaFuncSetAttribute(umma_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess) {
+      set_thread_error("umma conv: cannot raise dynamic shared memory limit"); cudaGetLastError(); return 2; }
+    ctx.attr_set = true;
+  }
   const int total = p.tiles_w * p.tiles_h * p.tiles_f * p.n_tiles;
   const int grid = total < ctx.num_sms ? total : ctx.num_sms;
-  umma_conv_kernel<<<grid, NUM_THREADS, SMEM_BYTES, s>>>(plan.tmap_a, plan.tmap_a2, plan.tmap_b, plan.tmap_a_lo, plan.tmap_a2_lo, plan.tmap_b_lo, p);
+  umma_conv_kernel<<<grid, NUM_THREADS, SMEM_BYTES, s>>>(plan.tmap_a, plan.tmap_b, plan.tmap_a_lo, plan.tmap_b_lo, p);
   SSNB_LAUNCH_CHECK("umma_conv_kernel");
   return 0;
 }

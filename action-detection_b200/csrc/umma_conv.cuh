@@ -24,35 +24,30 @@ struct UmmaContext {
 };
 
 struct UmmaConvParams {
-  int W, H, F;                    // spatial dims shared by input and output (stride-1 convolutions)
+  int W, H, F;                    // output dims; tiles enumerate output pixels (stride 1: the input has the same dims)
   int bw, bh, bf;                 // TMA box in pixels; bw*bh*bf <= 128 rows of the M tile
   int tiles_w, tiles_h, tiles_f;
   int n_tiles, block_n;           // N split of Cout
-  int stages, stage_bytes;        // smem pipeline depth / stride chosen from block_n
+  int stages, stage_bytes;        // first-generation kernel: smem pipeline depth / stride chosen from block_n
   int kchunks, ntaps, K;          // ceil(K/64), filter taps, reduction channels per tap
   int tap_dy[UMMA_MAX_TAPS], tap_dx[UMMA_MAX_TAPS];
   __half* out; int out_pitch, out_coff, Cout;
-  int out_stride, OH, OW;         // stride-2 layers: tiles run at input resolution, only even pixels are stored
-  int a_stride;                   // 2: tiles run at OUTPUT resolution and the A box uses TMA element stride 2
   const float* bias;              // [Cout] or nullptr
   int relu, accumulate;
   // horizontal fusion of sibling 1x1 convolutions (same input):
   int kchunks_a1, K1;             // K chunks [0, kchunks_a1) come from tmap_a (K1 real channels), the rest from tmap_a2
   int n_split;                    // output columns >= n_split go to out2 (second destination), else to out
   __half* out2; int out2_pitch, out2_coff;
-  // halo mode (3x3 stride-1 layers, conv1): ONE A box per K chunk covers the tile plus its filter halo, stored
-  // [y][frame][x][64 ch]; every tap is a shifted UMMA descriptor view into it (no per-tap re-staging of A)
-  int ablate;                     // timing experiments (SSNB_ABLATE bit mask): 1 no stores, 2 no bias loads, 4 empty epilogue, 8 no MMAs
-  int halo;
-  int pair;                       // CTA-pair kernel (cta_group::2): tiles are (N tile, pair of M tiles)
-  int v2;                         // second-generation kernel (umma_conv_v2.cu): warp-uniform role loops, grouped weight stages
+  // second-generation kernel (umma_conv_v2.cu, every stride-1 plan): ONE halo A box per K chunk covers the tile plus its
+  // filter halo, stored [y][frame][x][64 ch]; every tap is a shifted UMMA descriptor view into it.  CTA pairs
+  // (cta_group::2): tiles are (N tile, pair of M tiles)
+  int v2;                         // 1: launch umma_conv_v2_kernel; 0: the stride-2 forward kernel of umma_conv.cu
   int b_taps;                     // v2: taps per weight stage
-  int tiles_q;                    // v2: frame groups (pair mode: PAIRS of frame groups) = last digit of the tile walk
-  int epi_stages, epi_stage_bytes;// v2, experimental TMA-fed epilogue: ring depth (0 = off) and stride (old + activation chunk)
+  int tiles_q;                    // v2: PAIRS of frame groups = last digit of the tile walk
+  int epi_stages, epi_stage_bytes;// v2 TMA-fed epilogue: ring depth (0 = off) and stride (old + activation chunk)
   int a_stages, b_stages, a_stage_bytes, b_stage_bytes;
-  int a_loads, a_load_bytes;      // TMA loads per A stage (1: full halo box; >1: one box per horizontal shift)
+  int a_load_bytes;               // bytes the halo A box delivers
   int halo_x0, halo_y0;           // box origin relative to the tile origin (min dx, min dy)
-  int a_load_dx[4];               // extra W shift of each load
   int a_sbo;                      // bytes between consecutive 8-pixel row groups of a tap view
   int tap_aoff[UMMA_MAX_TAPS];    // byte offset of each tap's view inside the A stage
   // data gradient that is the LAST writer of its output: fuse dz = dy * (y > 0), y = activation of the same value
@@ -82,10 +77,10 @@ struct UmmaConvPlan {
   // SSNB_EXACT_TC mask fusion, applied only when launched with mask=true (see UmmaConvParams::mask32)
   const float* mask32 = nullptr; int mask32_pitch = 0, mask32_coff = 0;
   __half* mask_planes = nullptr; long long mask_planes_lo = 0; float mask_plane_scale = 1.0f; int* mask_flag = nullptr;
-  CUtensorMap tmap_old, tmap_y;   // experimental TMA-fed epilogue: output (old gradient) and mask-activation tiles, [128 rows][64 ch] boxes
+  CUtensorMap tmap_old, tmap_y;   // TMA-fed epilogue: output (old gradient) and mask-activation tiles, [128 rows][64 ch] boxes
   bool epi_maps_ready = false, epi_mask_ready = false;
   int epi_box[3] = {0, 0, 0}, epi_F = 0;     // box {W, F, H} extents and frame count for encoding tmap_y when the mask is attached
-  // geometry of the weight map (kept so that a variant can re-encode it with another box)
+  // geometry of the weight map (each kernel encodes it with its own box)
   const __half* b_ptr = nullptr; unsigned long long b_dims[3] = {0, 0, 0}, b_strides[2] = {0, 0};
   UmmaConvParams p;
 };
@@ -96,7 +91,7 @@ struct UmmaConvPlan {
 struct UmmaTcOpts { long long w_lo_off = 0; float* out32 = nullptr; float alpha = 1.0f; const float* alpha_dev = nullptr; float* out32_2 = nullptr; };
 void umma_context_init(UmmaContext& ctx, bool fp16);
 void umma_context_destroy(UmmaContext& ctx);
-// forward convolution plan (stride 1): in/out views, weights wd = [tap][cout][cin] fp16
+// forward convolution plan (stride 1, or stride 2 on the first-generation kernel): in/out views, weights wd = [tap][cout][cin] fp16
 int umma_conv_bind_fwd(UmmaContext& ctx, UmmaConvPlan& plan, View in, View out, int F, int cin, int cout, int k, int pad,
                        int stride, const __half* w_tap_n_k, const float* bias, const UmmaTcOpts* tc = nullptr);
 // generic tap table variant (conv1 in space-to-depth form: 16 taps of a 4x4 stride-1 convolution)
@@ -115,7 +110,7 @@ int umma_conv_launch(UmmaContext& ctx, const UmmaConvPlan& plan, cudaStream_t s,
 // second-generation kernel (umma_conv_v2.cu); `p` = plan.p with the per-launch fields (mask) already applied
 bool umma_conv_v2_supported(int ntaps);
 int umma_conv_v2_launch(UmmaContext& ctx, const UmmaConvPlan& plan, const UmmaConvParams& p, cudaStream_t s);
-void umma_conv_set_mask(UmmaContext& ctx, UmmaConvPlan& plan, View y);
+int umma_conv_set_mask(UmmaContext& ctx, UmmaConvPlan& plan, View y);
 // EXACT_TC: y32 = fp32 activation of the output value, dplanes = that value's gradient operand planes (hi base + lo_off)
 void umma_conv_set_mask_tc(UmmaConvPlan& plan, View y32, View dplanes, float plane_scale, int* flag);
 
@@ -138,8 +133,8 @@ struct UmmaWgradParams {
   float* bias_partial;            // [split][Cout] column sums of dz (bias gradient) from an extra ones-operand MMA, or nullptr
   int taps_per_cta, tap_groups, mma_n;   // taps sharing one dz tile per CTA; N of each tap's MMA
   int stages, stage_bytes;        // pipeline depth / stride
-  int halo;                       // x staged as one halo box per 64 channels; taps are descriptor views (tap_xoff)
-  int run_len, run_stride;        // halo: the CTA's taps are one run of equally spaced views taken by a single MMA (N = run_len*64)
+  int run_len, run_stride;        // run_len > 1: x staged as one halo box per 64 channels, the CTA's taps are one run of
+                                  // equally spaced descriptor views (tap_xoff, run_stride bytes apart) taken by a single MMA
   int x_box_bytes, x_box_tx, x_sbo, halo_x0, halo_y0, tap_xoff[UMMA_MAX_TAPS];   // box stride in smem / bytes one box delivers
   float* partial;
   int nseg;                       // 3: SSNB_EXACT_TC, every pixel tile runs (dz_lo, x_hi), (dz_hi, x_lo), (dz_hi, x_hi)

@@ -1,6 +1,6 @@
 // tcgen05 implicit-GEMM convolution, second generation (sm_100a): the role loops are written warp-uniformly.
 //
-// Measured on B200 (tools/ablate.sh): with the MMAs, the epilogue AND every TMA load removed, the first-generation
+// Measured on B200 (round 1, ablation runs): with the MMAs, the epilogue AND every TMA load removed, the first-generation
 // kernels (umma_conv.cu) still took 85-90 % of their full time -- the single-thread producer / MMA-issue loops
 // (divergent `if (lane == 0)` regions: vector registers, R2UR + vote loops around every UTMALDG / UTCHMMA, runtime
 // divisions per tile, dynamically indexed parameter arrays in local memory) bounded the kernel, not memory or the tensor
@@ -11,8 +11,8 @@
 //
 //   layout   halo A boxes (one per K chunk, [y][frame][x][64 ch], taps = shifted UMMA descriptor views; a 1x1 layer
 //            is the halo-free case), weight stages of G taps x rows x 64 ch
-//   PAIR     two CTAs of a cluster split two frame-adjacent M tiles and each stages half of the weight rows; the
-//            leader issues M = 256 cta_group::2 MMAs (umma_conv.cu has the protocol notes)
+//   pairs    two CTAs of a cluster split two frame-adjacent M tiles and each stages half of the weight rows; the
+//            leader issues M = 256 cta_group::2 MMAs
 //   warp 0   TMA producer, warp 1 MMA issuer, warps 2..9 epilogue (TMEM -> bias/ReLU or accumulate/mask -> fp16 NHWC)
 #include <cstdio>
 #include <cstdlib>
@@ -48,7 +48,7 @@ __device__ __forceinline__ bool elect_one() {
 }
 
 // Tile walk without divisions: digits (N tile, tile column, tile row, frame group) advance by the digits of the grid
-// stride with carries.  In PAIR mode the last digit counts PAIRS of frame groups and CTA `rank` owns group 2*mq + rank.
+// stride with carries.  The last digit counts PAIRS of frame groups and CTA `rank` of the pair owns group 2*mq + rank.
 struct TileIter {
   int nt, mw, mh, mq, sn, sw, sh, sq;
   __device__ __forceinline__ void init(const UmmaConvParams& p, int first, int step) {
@@ -63,15 +63,6 @@ struct TileIter {
     mq += sq + c;
   }
 };
-
-template <bool PAIR>
-__device__ __forceinline__ void commit_bar(uint64_t* bar) {
-  if (PAIR) umma_commit_pair(bar); else umma_commit(bar);
-}
-template <bool PAIR>
-__device__ __forceinline__ void mma_lohi(uint32_t d, uint32_t alo, uint32_t ahi, uint32_t blo, uint32_t bhi, uint32_t idesc, uint32_t acc) {
-  if (PAIR) umma_f16_lohi_pair(d, alo, ahi, blo, bhi, idesc, acc); else umma_f16_lohi(d, alo, ahi, blo, bhi, idesc, acc);
-}
 
 // one 16-column chunk of an accumulator row: bias / accumulate / ReLU / ReLU-gradient mask, fp16 store (32 bytes)
 template <bool HAS_BIAS>
@@ -106,20 +97,19 @@ __device__ __forceinline__ void store_chunk(const UmmaConvParams& p, const uint3
 #pragma unroll
     for (int j = 0; j < 8; ++j) q.v[j] &= __hgt2_mask(*reinterpret_cast<const __half2*>(&y.v[j]), zero);     // keep where y > 0 (NaN -> 0)
   }
-  if (p.ablate & 1) { if (v[0] == 12345.678f) stg256(dst, q); return; }     // SSNB_ABLATE=1: no stores
   stg256(dst, q);
 }
 
 // register budget: 10 warps on 4 sub-partitions = 3 warps on one of them, 16384 / (3 * 32) = 170 -> ptxas caps at 168
 // (a __maxnreg__(200) build compiles but cannot launch); two prefetch buffers fit, three spill
-// EPI selects the epilogue: 0 register-prefetch (forward; data gradients under SSNB_EPI_TMA=0); 2 TMA-fed (data gradients
-// that read the old gradient / the mask activation: an eleventh warp streams those tiles of every 64-column chunk into a
-// shared-memory ring with TMA, the epilogue warps read them with conflict-free LDS instead of scattered global loads;
-// validated and measured on B200 in round 2: -0.18 ms per training step).
+// EPI selects the epilogue: 0 register-prefetch (forward, and data gradients whose operand rings leave no room for the
+// epilogue ring); 2 TMA-fed (data gradients that read the old gradient / the mask activation: an eleventh warp streams
+// those tiles of every 64-column chunk into a shared-memory ring with TMA, the epilogue warps read them with
+// conflict-free LDS instead of scattered global loads; validated and measured on B200 in round 2: -0.18 ms per training step).
 // EPI == 3: SSNB_EXACT_TC.  The producer walks every K chunk three times -- (A_lo, B_hi), (A_hi, B_lo), (A_hi, B_hi): the
 // error-compensated fp16 product, ~22 significand bits per operand -- and the epilogue works in fp32 (out32 = alpha * acc
 // + bias, ReLU | + old) and emits the result's own hi / lo operand planes for the consuming convolutions.
-template <bool PAIR, int NTAPS, int EPI>
+template <int NTAPS, int EPI>
 __global__ void __launch_bounds__(EPI == 2 ? NUM_THREADS + 32 : NUM_THREADS, 1)
 umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a2,
                     const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_old,
@@ -144,10 +134,10 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   // warp index through a shuffle: provably warp-uniform, so the role branches below are uniform branches and the loop
   // state inside them can live in uniform registers
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x / 32), 0), lane = threadIdx.x % 32;
-  const uint32_t rank = PAIR ? cluster_ctarank() : 0u;
+  const uint32_t rank = cluster_ctarank();
   const bool leader = rank == 0;
-  const int first = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-  const int step = PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const int first = (int)(blockIdx.x >> 1);
+  const int step = (int)(gridDim.x >> 1);
   constexpr bool ONE_RING = NTAPS == 1;        // 1x1 layers: A box and weight slab of a step share one barrier pair
 
   // folded-BN bias of every output column of this launch, zero past Cout: the epilogue reads it with broadcast LDS
@@ -163,7 +153,7 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_b_lo)) : "memory");
     }
     for (int i = 0; i < MAX_STAGES; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 1); mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], (PAIR ? 2 : 1) * EPI_WARPS); }
+    for (int i = 0; i < 2; ++i) { mbar_init(&tfull_bar[i], 1); mbar_init(&tempty_bar[i], 2 * EPI_WARPS); }
     if (TMAE) {
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_old)) : "memory");
       asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmap_y)) : "memory");
@@ -172,22 +162,16 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 1) {
-    if (PAIR) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
   // Programmatic dependent launch: everything above (barrier init, tensor-map prefetch, TMEM allocation) touches nothing the
   // previous kernel of the stream produced, so it overlaps that kernel's tail; from here on its results are needed.
-  // (Both instructions are no-ops when the launch does not carry the programmatic-serialization attribute.)
   asm volatile("griddepcontrol.wait;" ::: "memory");
   if (p.bias)
     for (int i = threadIdx.x; i < p.n_tiles * p.block_n; i += (TMAE ? NUM_THREADS + 32 : NUM_THREADS)) bias_s[i] = i < p.Cout ? __ldg(p.bias + i) : 0.f;
   tc_fence_before();
-  if (PAIR) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   tc_fence_after();
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
@@ -197,14 +181,14 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     const bool el = elect_one();
     TileIter it; it.init(p, first, step);
     uint32_t as = 0, aph = 0, bs = 0, bph = 0;
-    const int rows_b = PAIR ? p.block_n / 2 : p.block_n;
-    const uint32_t a_tx = (PAIR ? 2u : 1u) * (uint32_t)(p.a_loads * p.a_load_bytes);
-    const uint32_t b_tx = (PAIR ? 2u : 1u) * (uint32_t)(rows_b * p.b_taps) * BLOCK_K * 2;
+    const int rows_b = p.block_n / 2;
+    const uint32_t a_tx = 2u * (uint32_t)p.a_load_bytes;           // both CTAs' boxes complete on the leader's barrier
+    const uint32_t b_tx = 2u * (uint32_t)(rows_b * p.b_taps) * BLOCK_K * 2;
     const int groups = NTAPS / p.b_taps;
     for (; it.valid(p); it.next(p)) {
       const int w0 = it.mw * p.bw + p.halo_x0, h0 = it.mh * p.bh + p.halo_y0;
-      const int f0 = (PAIR ? 2 * it.mq + (int)rank : it.mq) * p.bf;
-      const int n0 = it.nt * p.block_n + (PAIR ? (int)rank * rows_b : 0);
+      const int f0 = (2 * it.mq + (int)rank) * p.bf;
+      const int n0 = it.nt * p.block_n + (int)rank * rows_b;
       const int nseg = TC ? p.nseg : 1;
       for (int seg = 3 - nseg; seg < 3; ++seg)
       for (int kc = 0; kc < p.kchunks; ++kc) {
@@ -215,16 +199,10 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
           const bool src1 = kc < p.kchunks_a1;
           const CUtensorMap* map = (TC && seg == 0) ? (src1 ? &tmap_a_lo : &tmap_a2_lo) : (src1 ? &tmap_a : &tmap_a2);
           const int c0 = (src1 ? kc : kc - p.kchunks_a1) * BLOCK_K;
-          if (PAIR) {
-            if (leader) mbar_expect_tx(&a_full[as], ONE_RING ? a_tx + b_tx : a_tx);
-            const uint32_t bar = mapa_shared(smem_u32(&a_full[as]), 0);
-            for (int l = 0; l < p.a_loads; ++l) tma_load_4d_pair(sa + l * p.a_load_bytes, map, bar, c0, w0 + p.a_load_dx[l], f0, h0);
-            if (ONE_RING) tma_load_3d_pair(smem_b + as * p.b_stage_bytes, bmap, bar, kc * BLOCK_K, n0, 0);
-          } else {
-            mbar_expect_tx(&a_full[as], ONE_RING ? a_tx + b_tx : a_tx);
-            for (int l = 0; l < p.a_loads; ++l) tma_load_4d(sa + l * p.a_load_bytes, map, &a_full[as], c0, w0 + p.a_load_dx[l], f0, h0);
-            if (ONE_RING) tma_load_3d(smem_b + as * p.b_stage_bytes, bmap, &a_full[as], kc * BLOCK_K, n0, 0);
-          }
+          if (leader) mbar_expect_tx(&a_full[as], ONE_RING ? a_tx + b_tx : a_tx);
+          const uint32_t bar = mapa_shared(smem_u32(&a_full[as]), 0);
+          tma_load_4d_pair(sa, map, bar, c0, w0, f0, h0);
+          if (ONE_RING) tma_load_3d_pair(smem_b + as * p.b_stage_bytes, bmap, bar, kc * BLOCK_K, n0, 0);
         }
         if (++as == (uint32_t)p.a_stages) { as = 0; aph ^= 1; }
         if (!ONE_RING) {
@@ -232,13 +210,8 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             mbar_wait(&b_empty[bs], bph ^ 1);
             if (el) {
               uint8_t* sb = smem_b + bs * p.b_stage_bytes;
-              if (PAIR) {
-                if (leader) mbar_expect_tx(&b_full[bs], b_tx);
-                tma_load_3d_pair(sb, bmap, mapa_shared(smem_u32(&b_full[bs]), 0), kc * BLOCK_K, n0, g * p.b_taps);
-              } else {
-                mbar_expect_tx(&b_full[bs], b_tx);
-                tma_load_3d(sb, bmap, &b_full[bs], kc * BLOCK_K, n0, g * p.b_taps);
-              }
+              if (leader) mbar_expect_tx(&b_full[bs], b_tx);
+              tma_load_3d_pair(sb, bmap, mapa_shared(smem_u32(&b_full[bs]), 0), kc * BLOCK_K, n0, g * p.b_taps);
             }
             if (++bs == (uint32_t)p.b_stages) { bs = 0; bph ^= 1; }
           }
@@ -246,13 +219,13 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       }
     }
   } else if (warp == 1) {
-    // ===== MMA issuer (whole warp walks the pipeline; one elected lane issues; PAIR: leader CTA only) =====
-    if (!PAIR || leader) {
+    // ===== MMA issuer (whole warp walks the pipeline; one elected lane issues; leader CTA of the pair only) =====
+    if (leader) {
       const bool el = elect_one();
-      const uint32_t idesc = make_idesc_f16_m(PAIR ? 256 : 128, p.block_n);
+      const uint32_t idesc = make_idesc_f16_m(256, p.block_n);
       const uint32_t a_hi = desc_hi_sw128(p.a_sbo), b_hi = desc_hi_sw128(1024);
       const uint32_t a_stage_lo = (uint32_t)p.a_stage_bytes >> 4, b_stage_lo = (uint32_t)p.b_stage_bytes >> 4;
-      const uint32_t slab_lo = (uint32_t)((PAIR ? p.block_n / 2 : p.block_n) * BLOCK_K * 2) >> 4;     // one tap inside a weight stage
+      const uint32_t slab_lo = (uint32_t)(p.block_n / 2 * BLOCK_K * 2) >> 4;     // one tap inside a weight stage
       const uint32_t a_base = desc_lo(smem_u32(smem)), b_base = desc_lo(smem_u32(smem_b));
       const int btaps = p.b_taps;
       uint32_t as = 0, aph = 0, bs = 0, bph = 0, acc = 0, acc_phase = 0;
@@ -278,23 +251,23 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
               tc_fence_after();
               b_lo = b_base + bs * b_stage_lo;
             }
-            if (el && !(p.ablate & 8)) {
+            if (el) {
               const uint32_t a_lo = a_lo0 + ((uint32_t)p.tap_aoff[tap] >> 4);
 #pragma unroll
               for (int k = 0; k < BLOCK_K / UMMA_K; ++k)
-                if (k < nk) mma_lohi<PAIR>(d_tmem, a_lo + 2 * k, a_hi, b_lo + 2 * k, b_hi, idesc, (seg | kc | tap | k) ? 1u : 0u);
+                if (k < nk) umma_f16_lohi_pair(d_tmem, a_lo + 2 * k, a_hi, b_lo + 2 * k, b_hi, idesc, (seg | kc | tap | k) ? 1u : 0u);
             }
             b_lo += slab_lo;
             if (!ONE_RING && ++gi == btaps) {
               gi = 0;
-              if (el) commit_bar<PAIR>(&b_empty[bs]);
+              if (el) umma_commit_pair(&b_empty[bs]);
               if (++bs == (uint32_t)p.b_stages) { bs = 0; bph ^= 1; }
             }
           }
-          if (el) commit_bar<PAIR>(&a_empty[as]);
+          if (el) umma_commit_pair(&a_empty[as]);
           if (++as == (uint32_t)p.a_stages) { as = 0; aph ^= 1; }
         }
-        if (el) commit_bar<PAIR>(&tfull_bar[acc]);
+        if (el) umma_commit_pair(&tfull_bar[acc]);
         __syncwarp();
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
       }
@@ -314,14 +287,13 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     // training step -- and removed; see profiles/README.md.)
     for (; it.valid(p); it.next(p)) {
       const int w = it.mw * p.bw + rw, h = it.mh * p.bh + rh;
-      const int f = (PAIR ? 2 * it.mq + (int)rank : it.mq) * p.bf + rf;
+      const int f = (2 * it.mq + (int)rank) * p.bf + rf;
       const int n0 = it.nt * p.block_n;
       const bool valid = (rh < p.bh) && (w < p.W) && (h < p.H) && (f < p.F);
-      const long long opix = (long long)(f * p.OH + h) * p.OW + w;
+      const long long opix = (long long)(f * p.H + h) * p.W + w;
       __half* orow = p.out + opix * p.out_pitch + p.out_coff;
       __half* orow2 = p.out2 + opix * p.out2_pitch + p.out2_coff - p.n_split;
       const __half* mrow = p.mask_y ? p.mask_y + opix * p.mask_pitch + p.mask_coff : nullptr;
-      const int ncol = (p.ablate & 4) ? 0 : p.block_n;              // SSNB_ABLATE=4 (timing experiment): empty epilogue
       // Global operands of the epilogue (old gradient to accumulate into, activation for the ReLU-gradient mask) are
       // software-pipelined: the loads of column group i+1 go out before group i is processed, and those of a tile's
       // first group before the wait for its accumulator, so their DRAM/L2 latency overlaps the MMAs and the TMEM reads.
@@ -351,14 +323,12 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         mbar_wait(&tfull_bar[acc], acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + acc * 256 + ((uint32_t)(quad * 32) << 16);
-        if (cpar * 32 >= ncol) {                                    // narrow tile: this warp has no columns, release at once
+        if (cpar * 32 >= p.block_n) {                                    // narrow tile: this warp has no columns, release at once
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) {
-            if (PAIR) mbar_arrive_cluster(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]);
-          }
+          if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);
         }
-        for (int c0 = cpar * 32; c0 < ncol; c0 += 64) {
+        for (int c0 = cpar * 32; c0 < p.block_n; c0 += 64) {
           const bool two = c0 + 16 < p.block_n;                     // warp-uniform
           const int cola = n0 + c0, colb = cola + 16;
           uint32_t ra[16], rb[16];
@@ -368,9 +338,7 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
           if (c0 + 64 >= p.block_n) {                               // last TMEM read of this tile: hand the accumulator back early
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) {
-              if (PAIR) mbar_arrive_cluster(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]);
-            }
+            if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);
           }
           if (valid && cola < p.Cout) {
             const bool d1 = cola < p.n_split;
@@ -389,12 +357,10 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         mbar_wait(&tfull_bar[acc], acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + acc * 256 + ((uint32_t)(quad * 32) << 16);
-        if (cpar * 32 >= ncol) {                                    // narrow tile: this warp has no columns, release at once
+        if (cpar * 32 >= p.block_n) {                                    // narrow tile: this warp has no columns, release at once
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) {
-            if (PAIR) mbar_arrive_cluster(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]);
-          }
+          if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);
         }
         const int nchunks = (p.block_n + 63) / 64;
         for (int i = 0; i < nchunks; ++i) {
@@ -413,7 +379,7 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
           __syncwarp();
           if (lane == 0) mbar_arrive(&e_empty[es]);                 // release semantics order the shared loads above before it
           if (++es == (uint32_t)p.epi_stages) { es = 0; eph ^= 1; }
-          if (c0 < ncol) {
+          if (c0 < p.block_n) {
             const bool two = c0 + 16 < p.block_n;                   // warp-uniform
             const int cola = n0 + c0, colb = cola + 16;
             const bool va = valid && cola < p.Cout, vb = two && valid && colb < p.Cout;
@@ -425,9 +391,7 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             if (c0 + 64 >= p.block_n) {                             // last TMEM read of this tile: hand the accumulator back early
               tc_fence_before();
               __syncwarp();
-              if (lane == 0) {
-                if (PAIR) mbar_arrive_cluster(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]);
-              }
+              if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);
             }
             if (va) store_chunk<false>(p, ra, ba, orow + cola, oa, ya);
             if (vb) store_chunk<false>(p, rb, bb, orow + colb, ob, yb);
@@ -437,29 +401,27 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         // two rotating prefetch buffers (a third spills under the 168-register cap: measured no faster)
         constexpr int NB = 2;
         Pre pp[NB] = {};                                               // indices are compile-time after unrolling: no register copies
-        if (cpar * 32 < ncol) prefetch(cpar * 32, pp[0]);
+        if (cpar * 32 < p.block_n) prefetch(cpar * 32, pp[0]);
         mbar_wait(&tfull_bar[acc], acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + acc * 256 + ((uint32_t)(quad * 32) << 16);
-        if (cpar * 32 >= ncol) {                                      // narrow tile: this warp has no columns, release at once
+        if (cpar * 32 >= p.block_n) {                                      // narrow tile: this warp has no columns, release at once
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) {
-            if (PAIR) mbar_arrive_cluster(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]);
-          }
+          if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);
         }
-        for (int cbase = cpar * 32; cbase < ncol; cbase += 64 * NB) {
+        for (int cbase = cpar * 32; cbase < p.block_n; cbase += 64 * NB) {
   #pragma unroll
           for (int u = 0; u < NB; ++u) {
             const int c0 = cbase + 64 * u;
-            if (c0 < ncol) {
+            if (c0 < p.block_n) {
               // one 32-column group: prefetch the operands of a later group, then TMEM -> registers -> epilogue math
               const bool two = c0 + 16 < p.block_n;                   // warp-uniform
               const int cola = n0 + c0, colb = cola + 16;
               const bool va = valid && cola < p.Cout, vb = two && valid && colb < p.Cout;
               __half* da = (cola < p.n_split ? orow : orow2) + cola;
               __half* db2 = (colb < p.n_split ? orow : orow2) + colb;
-              if (c0 + 64 * (NB - 1) < ncol) prefetch(c0 + 64 * (NB - 1), pp[(u + NB - 1) % NB]);
+              if (c0 + 64 * (NB - 1) < p.block_n) prefetch(c0 + 64 * (NB - 1), pp[(u + NB - 1) % NB]);
               float4 ba[4], bb[4];
               if (p.bias) {
   #pragma unroll
@@ -475,9 +437,7 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
               if (c0 + 64 >= p.block_n) {                             // last TMEM read of this tile: hand the accumulator back early
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) {
-                  if (PAIR) mbar_arrive_cluster(&tempty_bar[acc], 0); else mbar_arrive(&tempty_bar[acc]);
-                }
+                if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);
               }
               if (va) store_chunk<true>(p, ra, ba, da, pp[u].oa, pp[u].ya);
               if (vb) store_chunk<true>(p, rb, bb, db2, pp[u].ob, pp[u].yb);
@@ -497,7 +457,7 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
     TileIter it; it.init(p, first, step);
     for (; it.valid(p); it.next(p)) {
       const int w0 = it.mw * p.bw, h0 = it.mh * p.bh;
-      const int f0 = (PAIR ? 2 * it.mq + (int)rank : it.mq) * p.bf;
+      const int f0 = (2 * it.mq + (int)rank) * p.bf;
       const int n0 = it.nt * p.block_n;
       for (int i = 0; i < nchunks; ++i) {
         mbar_wait(&e_empty[es], eph ^ 1);
@@ -517,18 +477,17 @@ umma_conv_v2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   }
 
   tc_fence_before();
-  if (PAIR) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   if (warp == 1) {
     tc_fence_after();
-    if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS) : "memory");
   }
 }
 
-template <bool PAIR, int NTAPS, int EPI>
+template <int NTAPS, int EPI>
 int launch_one(const UmmaConvPlan& plan, const UmmaConvParams& p, int num_sms, cudaStream_t s) {
   static bool attr_set[64] = {};          // function attributes are per device
-  auto kern = umma_conv_v2_kernel<PAIR, NTAPS, EPI>;
+  auto kern = umma_conv_v2_kernel<NTAPS, EPI>;
   int dev = 0;
   cudaGetDevice(&dev);
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
@@ -539,34 +498,27 @@ int launch_one(const UmmaConvPlan& plan, const UmmaConvParams& p, int num_sms, c
   const int total = p.n_tiles * p.tiles_w * p.tiles_h * p.tiles_q;
   cudaLaunchConfig_t cfg = {};
   cudaLaunchAttribute attr[2];
-  int na = 0;
   cfg.blockDim = dim3(EPI == 2 ? NUM_THREADS + 32 : NUM_THREADS);
   cfg.dynamicSmemBytes = SMEM_BYTES;
   cfg.stream = s;
-  if (PAIR) {
-    const int pairs = std::min(total, num_sms / 2);
-    cfg.gridDim = dim3(2 * pairs);
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = 2; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-    ++na;
-  } else {
-    cfg.gridDim = dim3(std::min(total, num_sms));
-  }
-  // programmatic dependent launch (SSNB_PDL=0 turns it off): this kernel's prologue may overlap the previous kernel's tail
-  static const bool pdl = [] { const char* e = getenv("SSNB_PDL"); return !(e && e[0] == '0'); }();
-  if (pdl) { attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[na].val.programmaticStreamSerializationAllowed = 1; ++na; }
-  cfg.attrs = na ? attr : nullptr; cfg.numAttrs = na;
+  const int pairs = std::min(total, num_sms / 2);
+  cfg.gridDim = dim3(2 * pairs);
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  // programmatic dependent launch: this kernel's prologue may overlap the previous kernel's tail
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = 2;
   if (cudaLaunchKernelEx(&cfg, kern, plan.tmap_a, plan.tmap_a2, plan.tmap_b, plan.tmap_old, plan.tmap_y, plan.tmap_a_lo, plan.tmap_a2_lo,
                          plan.tmap_b_lo, p) != cudaSuccess) {
     set_thread_error(std::string("umma_conv_v2_kernel launch: ") + cudaGetErrorString(cudaGetLastError())); return 2; }
   return 0;
 }
 
-template <bool PAIR, int EPI>
+template <int EPI>
 int launch_taps(const UmmaConvPlan& plan, const UmmaConvParams& p, int num_sms, cudaStream_t s) {
-  if (p.ntaps == 1) return launch_one<PAIR, 1, EPI>(plan, p, num_sms, s);
-  if (p.ntaps == 4) return launch_one<PAIR, 4, EPI>(plan, p, num_sms, s);
-  return launch_one<PAIR, 9, EPI>(plan, p, num_sms, s);
+  if (p.ntaps == 1) return launch_one<1, EPI>(plan, p, num_sms, s);
+  if (p.ntaps == 4) return launch_one<4, EPI>(plan, p, num_sms, s);
+  return launch_one<9, EPI>(plan, p, num_sms, s);
 }
 
 }  // namespace
@@ -579,10 +531,8 @@ int umma_conv_v2_launch(UmmaContext& ctx, const UmmaConvPlan& plan, const UmmaCo
   const bool reads = !p.bias && !p.relu && (p.accumulate || p.mask_y);
   const int epi = p.out_f32 ? 3 : ((reads && p.epi_stages > 0 && plan.epi_maps_ready && (!p.mask_y || plan.epi_mask_ready)) ? 2 : 0);
   if (p.out_f32 && p.mask_y) { set_thread_error("umma conv v2: the fp32 epilogue takes its mask through mask32"); return 3; }
-  int rc;
-  if (epi == 3) rc = p.pair ? launch_taps<true, 3>(plan, p, ctx.num_sms, s) : launch_taps<false, 3>(plan, p, ctx.num_sms, s);
-  else if (p.pair) rc = epi == 2 ? launch_taps<true, 2>(plan, p, ctx.num_sms, s) : launch_taps<true, 0>(plan, p, ctx.num_sms, s);
-  else rc = epi == 2 ? launch_taps<false, 2>(plan, p, ctx.num_sms, s) : launch_taps<false, 0>(plan, p, ctx.num_sms, s);
+  const int rc = epi == 3 ? launch_taps<3>(plan, p, ctx.num_sms, s)
+               : epi == 2 ? launch_taps<2>(plan, p, ctx.num_sms, s) : launch_taps<0>(plan, p, ctx.num_sms, s);
   if (rc) return rc;
   SSNB_LAUNCH_CHECK("umma_conv_v2_kernel");
   return 0;

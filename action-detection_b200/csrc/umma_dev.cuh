@@ -70,19 +70,6 @@ __device__ __forceinline__ uint64_t make_desc_k_sw128(uint32_t saddr) {
   return d;
 }
 
-// same, for a view into a larger (halo) tile: `sbo_bytes` between 8-row groups, start not necessarily 1024-byte
-// aligned (base_offset = descriptor bits [49,52), the row phase of the start address inside the swizzle atom)
-__device__ __forceinline__ uint64_t make_desc_k_sw128_view(uint32_t saddr, uint32_t sbo_bytes, uint32_t base_off) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)(base_off & 7) << 49;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-
 // instruction descriptor, kind::f16: D=f32, A=B=f16, both K-major, M=128, N=n
 __device__ __forceinline__ uint32_t make_idesc_f16(int n) {
   return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BLOCK_M >> 4) << 24);
@@ -191,18 +178,6 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-
-// MN-major, SWIZZLE_128B descriptor: tile stored as [k rows][64 MN elements = 128 B]; 8-row groups
-// every 1024 B (SBO), next 64-element MN atom every `lbo_bytes` (LBO).
-__device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t saddr, uint32_t lbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
 // kind::f16 instruction descriptor with both operands MN-major (a_major bit 15, b_major bit 16)
 __device__ __forceinline__ uint32_t make_idesc_f16_mn(int n) {
   return (1u << 4) | (1u << 15) | (1u << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BLOCK_M >> 4) << 24);

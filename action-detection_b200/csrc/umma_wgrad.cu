@@ -54,6 +54,7 @@ umma_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_cons
   const int pt0 = split * p.ptiles_per_split;
   const int pt1 = min(pt0 + p.ptiles_per_split, ptiles);
   const int nboxes_b = p.block_n / 64;
+  const bool run = p.run_len > 1;                  // halo x box, the CTA's taps taken by one MMA (see umma_wgrad_bind_taps)
   // CTAs of the first input tile / tap group also reduce dz over pixels: db[co] = sum_p dz[p, co] = dz^T * 1
   const bool do_bias = p.bias_partial != nullptr && nt == 0 && tgrp == 0;
   const int bias_col = p.taps_per_cta * p.mma_n;
@@ -86,7 +87,7 @@ umma_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_cons
   if (warp == 0) {
     const bool el = elect_one_lane();
     uint32_t stage = 0, phase = 0;
-    const uint32_t tx_bytes = p.halo ? (uint32_t)(2 * BOX_BYTES + nboxes_b * p.x_box_tx) : (uint32_t)(2 + nboxes_b * ntap) * BOX_BYTES;
+    const uint32_t tx_bytes = run ? (uint32_t)(2 * BOX_BYTES + nboxes_b * p.x_box_tx) : (uint32_t)(2 + nboxes_b * ntap) * BOX_BYTES;
     // pixel-tile coordinates advance by carries (no divisions in the loop)
     int tw = pt0 % p.tiles_w, th = (pt0 / p.tiles_w) % p.tiles_h, tf = pt0 / (p.tiles_w * p.tiles_h);
     for (int pt = pt0; pt < pt1; ++pt) {
@@ -100,7 +101,7 @@ umma_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_cons
         uint8_t* sa = smem + stage * STAGE_BYTES;
         uint8_t* sb = sa + A_BYTES;
         mbar_expect_tx(&full_bar[stage], tx_bytes);
-        if (p.halo) {
+        if (run) {
           // halo layout: tensor-map dims {C, W, F, H}; ONE x box per 64 input channels covers the tile plus the filter
           // border, every tap of this CTA is a shifted descriptor view into it
           tma_load_4d(sa, mdz, &full_bar[stage], m0, w0, f0, h0);
@@ -129,21 +130,19 @@ umma_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_cons
     const uint32_t base_lo = ((smem_u32(smem) >> 4) & 0x3FFF) | lbo;
     const uint32_t ones_lo = ((smem_u32(smem + ONES_OFF) >> 4) & 0x3FFF) | lbo;
     const uint32_t kstep_lo = (UMMA_K * 128) >> 4;                    // 16 pixel rows
-    // x operand: classic = one [64 px][64 ch] box per (tap, 64 channels); halo = views into the halo box: 8-pixel row
-    // groups x_sbo bytes apart, 64-channel atoms x_box_bytes apart
-    const uint32_t hi_x = p.halo ? desc_hi_sw128(p.x_sbo) : hi;
-    const uint32_t lbo_x = p.halo ? ((uint32_t)((p.x_box_bytes >> 4) & 0x3FFF) << 16) : lbo;
-    const uint32_t kstep_x = p.halo ? (uint32_t)(2 * p.x_sbo) >> 4 : kstep_lo;
+    // x operand of a tap run: views into the halo box, 8-pixel row groups x_sbo bytes apart
+    const uint32_t hi_x = desc_hi_sw128(p.x_sbo);
+    const uint32_t kstep_x = (uint32_t)(2 * p.x_sbo) >> 4;
     uint32_t stage = 0, phase = 0;
     for (int pt = pt0; pt < pt1; ++pt)
     for (int seg = 3 - p.nseg; seg < 3; ++seg) {
       mbar_wait(&full_bar[stage], phase);
       tc_fence_after();
       const uint32_t sa_lo = base_lo + stage * ((uint32_t)STAGE_BYTES >> 4);
-      const uint32_t sb_lo = ((sa_lo + (A_BYTES >> 4)) & 0xFFFFu) | lbo_x;
+      const uint32_t sb_lo = ((sa_lo + (A_BYTES >> 4)) & 0xFFFFu) | lbo;
       if (el) {
         const uint32_t first = (pt > pt0 || seg > 3 - p.nseg) ? 1u : 0u;
-        if (p.run_len > 1) {
+        if (run) {
           // the taps of this CTA form ONE run whose views are `run_stride` bytes apart: a single MMA takes them as
           // consecutive 64-channel N atoms (LBO = run_stride), so the dz tile is read once per K step instead of once
           // per tap (the kernel is bound by those shared-memory reads)
@@ -152,12 +151,13 @@ umma_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dz, const __grid_cons
           for (int k = 0; k < 64 / UMMA_K; ++k)
             umma_f16_lohi(tmem_base, sa_lo + k * kstep_lo, hi, xb_lo + k * kstep_x, hi_x, idesc_run, first | (uint32_t)k);
         } else {
-        for (int t = 0; t < ntap; ++t) {
-          const uint32_t xb_lo = sb_lo + (p.halo ? (uint32_t)p.tap_xoff[tap0 + t] >> 4 : (uint32_t)(t * nboxes_b) * (BOX_BYTES >> 4));
+          // classic layout: one [64 px][64 ch] box per (tap, 64 channels)
+          for (int t = 0; t < ntap; ++t) {
+            const uint32_t xb_lo = sb_lo + (uint32_t)(t * nboxes_b) * (BOX_BYTES >> 4);
 #pragma unroll
-          for (int k = 0; k < 64 / UMMA_K; ++k)      // 16 pixel rows (2 groups of 8) per instruction
-            umma_f16_lohi(tmem_base + t * p.mma_n, sa_lo + k * kstep_lo, hi, xb_lo + k * kstep_x, hi_x, idesc, first | (uint32_t)k);
-        }
+            for (int k = 0; k < 64 / UMMA_K; ++k)      // 16 pixel rows (2 groups of 8) per instruction
+              umma_f16_lohi(tmem_base + t * p.mma_n, sa_lo + k * kstep_lo, hi, xb_lo + k * kstep_lo, hi, idesc, first | (uint32_t)k);
+          }
         }
         if (do_bias && seg != 1) {          // column sums of dz: hi and lo planes once each (seg 1 re-stages dz_hi against x_lo)
 #pragma unroll
@@ -246,26 +246,21 @@ int umma_wgrad_bind_taps(UmmaContext& ctx, UmmaWgradPlan& plan, View dz, View x,
   // the accumulators (taps * mma_n fp32 columns) must fit the 512 TMEM columns
   p.mma_n = p.block_n;
   if (p.n_tiles == 1 && cin < p.block_n) p.mma_n = (cin + 15) / 16 * 16;     // narrow inputs (conv1 space-to-depth: 16)
-  // halo variant (stride-1 multi-tap layers): ONE x box per 64 input channels covers the 64-pixel tile plus the filter
-  // border ([y][frame][x] pixel order, as in umma_conv_v2.cu) and every tap is a shifted descriptor view into it.
-  // Default: only where a whole ROW of taps can then be taken by a single MMA -- 64-channel layers, whose tap views are
-  // equally spaced, so they are consecutive 64-channel N atoms with LBO = the tap spacing (128 B for a 3x3 row, 1 KiB
-  // for conv1's four vertical taps).  That reads the 4 KiB dz tile once per K step instead of once per tap, which is
-  // what bounds this kernel (shared-memory bandwidth): conv2_3x3 283 -> 163 us, conv1 254 -> 148 us.  Without the
-  // fusion the halo layout is SLOWER than per-tap boxes (more taps per CTA, same dz re-reads: 3.7 vs 2.9 ms over the
-  // 69 layers), so wider layers keep the classic layout.  SSNB_WGRAD_HALO=0 off, 1 halo everywhere without fusion,
-  // 2 halo everywhere + fusion where possible.
+  // Tap runs (stride-1 multi-tap 64-channel layers): ONE x box per 64 input channels covers the 64-pixel tile plus the
+  // filter border ([y][frame][x] pixel order, as in umma_conv_v2.cu) and every tap is a shifted descriptor view into it.
+  // Where the views of a whole ROW of taps are equally spaced they are consecutive 64-channel N atoms with LBO = the tap
+  // spacing (128 B for a 3x3 row, 1 KiB for conv1's four vertical taps), so a single MMA takes the run.  That reads the
+  // 4 KiB dz tile once per K step instead of once per tap, which is what bounds this kernel (shared-memory bandwidth):
+  // conv2_3x3 283 -> 163 us, conv1 254 -> 148 us.  Without the run the halo layout is SLOWER than per-tap boxes (more
+  // taps per CTA, same dz re-reads: 3.7 vs 2.9 ms over the 69 layers), so every other layer keeps the classic layout.
   int x0 = 0, x1 = 0, y0 = 0, y1 = 0;
   for (int t = 0; t < ntaps; ++t) { x0 = std::min(x0, tdx[t]); x1 = std::max(x1, tdx[t]); y0 = std::min(y0, tdy[t]); y1 = std::max(y1, tdy[t]); }
-  const char* he = getenv("SSNB_WGRAD_HALO");
-  const int hmode = he ? atoi(he) : 3;                  // 3 = default: halo only with run fusion
-  bool halo = hmode != 0 && x_stride == 1 && ntaps > 1 && dz.W >= 7;
+  int hbh = 8;
+  while (hbh > 1 && dz.H % hbh) hbh >>= 1;
+  const int hbw = 8, hbf = 64 / (hbw * hbh), pw = hbw + (x1 - x0);
+  auto off = [&](int t) { return ((tdy[t] - y0) * hbf * pw + (tdx[t] - x0)) * 128; };
   int run_len = 1, run_stride = 0;
-  if (halo && hmode >= 2 && p.block_n == 64 && p.mma_n == 64) {
-    const int pw0 = 8 + (x1 - x0);
-    int hb = 8; while (hb > 1 && dz.H % hb) hb >>= 1;
-    const int hf = 64 / (8 * hb);
-    auto off = [&](int t) { return ((tdy[t] - y0) * hf * pw0 + (tdx[t] - x0)) * 128; };
+  if (x_stride == 1 && ntaps > 1 && dz.W >= 7 && p.block_n == 64 && p.mma_n == 64) {
     for (int r = 4; r >= 2; --r) {                      // longest run length (N = r*64 <= 256) that tiles the tap list evenly
       if (ntaps % r) continue;
       bool ok = true;
@@ -275,23 +270,15 @@ int umma_wgrad_bind_taps(UmmaContext& ctx, UmmaWgradPlan& plan, View dz, View x,
       if (ok && st > 0 && st % 16 == 0) { run_len = r; run_stride = st; break; }
     }
   }
-  if (hmode == 3 && run_len == 1) halo = false;
-  int hbw = 8, hbh = 8, hbf = 1, pw = 8, x_box = 0, h_taps = 1, h_stages = 0;
-  if (halo) {
-    while (hbh > 1 && dz.H % hbh) hbh >>= 1;
-    hbf = 64 / (hbw * hbh);
-    pw = hbw + (x1 - x0);
-    x_box = (pw * hbf * (hbh + (y1 - y0)) * 128 + 1023) / 1024 * 1024;
-    h_taps = run_len > 1 ? run_len : std::min(ntaps, (512 - 16) / p.mma_n);
-    h_stages = std::min(MAX_STAGES, PIPE_BYTES / (A_BYTES + (p.block_n / 64) * x_box));
-    if (h_taps < 2 || h_stages < 3) halo = false;
-  }
-  p.halo = halo ? 1 : 0;
-  p.run_len = halo ? run_len : 1; p.run_stride = run_stride;
+  const int x_box = (pw * hbf * (hbh + (y1 - y0)) * 128 + 1023) / 1024 * 1024;
+  const int h_stages = std::min(MAX_STAGES, PIPE_BYTES / (A_BYTES + (p.block_n / 64) * x_box));
+  if (h_stages < 3) run_len = 1;                        // the halo boxes leave too few stages: per-tap boxes
+  const bool halo = run_len > 1;
+  p.run_len = run_len; p.run_stride = run_stride;
   if (halo) {
     p.bw = hbw; p.bh = hbh; p.bf = hbf;
     p.tiles_w = (dz.W + hbw - 1) / hbw; p.tiles_h = dz.H / hbh; p.tiles_f = (F + hbf - 1) / hbf;
-    p.taps_per_cta = h_taps;
+    p.taps_per_cta = run_len;
     p.x_box_bytes = x_box; p.x_box_tx = pw * hbf * (hbh + (y1 - y0)) * 128; p.x_sbo = pw * 128; p.halo_x0 = x0; p.halo_y0 = y0;
     p.stage_bytes = A_BYTES + (p.block_n / 64) * x_box; p.stages = h_stages;
     for (int t = 0; t < ntaps; ++t) p.tap_xoff[t] = ((tdy[t] - y0) * hbf * pw + (tdx[t] - x0)) * 128;
@@ -311,8 +298,7 @@ int umma_wgrad_bind_taps(UmmaContext& ctx, UmmaWgradPlan& plan, View dz, View x,
   // one CTA per SM is resident (192 KiB pipeline), so a second wave only runs after the first: ONE wave of CTAs with
   // twice the pixels each does the same work with half the split-K partial traffic (every CTA writes its whole
   // 128 x taps*N fp32 accumulator: 100-250 KB) and no wave tail (conv2_3x3 used to run 300 CTAs = three waves)
-  const char* we = getenv("SSNB_WGRAD_WAVES");
-  int splits = ((we ? atoi(we) : 1) * ctx.num_sms) / ctas;
+  int splits = ctx.num_sms / ctas;
   if (splits < 1) splits = 1;
   if (splits > max_splits) splits = max_splits;
   if (splits > ptiles) splits = ptiles;
@@ -378,8 +364,9 @@ int umma_wgrad_launch(UmmaContext& ctx, const UmmaWgradPlan& plan, cudaStream_t 
   cfg.blockDim = dim3(NUM_THREADS);
   cfg.dynamicSmemBytes = SMEM_BYTES;
   cfg.stream = s;
-  static const bool pdl = [] { const char* e = getenv("SSNB_PDL"); return !(e && e[0] == '0'); }();
-  if (pdl) { attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[0].val.programmaticStreamSerializationAllowed = 1; cfg.attrs = attr; cfg.numAttrs = 1; }
+  // programmatic dependent launch: the kernel's prologue may overlap the previous kernel's tail
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
   if (cudaLaunchKernelEx(&cfg, umma_wgrad_kernel, plan.tmap_dz, plan.tmap_x, plan.tmap_dz_lo, plan.tmap_x_lo, p) != cudaSuccess) {
     set_thread_error(std::string("umma_wgrad_kernel launch: ") + cudaGetErrorString(cudaGetLastError())); return 2; }
   SSNB_LAUNCH_CHECK("umma_wgrad_kernel");
